@@ -39,6 +39,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the source tree as it found it (it may be read-only)
 
 METRIC = "env_steps_per_sec"
 UNIT = "env-steps/s"
@@ -74,7 +75,16 @@ def parse():
                          "is the nominal value times U(1-j, 1+j) (BASELINE.json configs[2])")
     ap.add_argument("--stats-every", type=int, default=16,
                     help="N>1: all-reduce the 64 B episode-statistics vector every this many bench steps")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (obs, reward, done) and "
+                         "the env state it left, for a fixed seeded sample of envs, as DIR/<name>.npy "
+                         "(float32/float64, at most 64 MB in all; rank r of several writes <name>_rank<r>.npy)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
 
 
 def workload_config(args, world):
@@ -89,6 +99,26 @@ def workload_config(args, world):
         "l2": "per-step action/obs/reward streams (>=750 MB) exceed the 126 MB L2; env state "
               "(3 MB) lives in registers across the whole launch",
     }
+
+
+DUMP_BYTES = 60 << 20   # --dump-outputs: array bytes of all ranks together (files under 64 MB)
+
+
+def sample_outputs(batch, out, budget):
+    """Host copies of what the last rollout returned -- obs [T, obs_dim, k], reward [T, k], done flags [T, k]
+    (as float32) -- and of the env state [n_state, k] it left, for k envs drawn with a fixed seed: all of them
+    when they fit in `budget` bytes."""
+    import numpy as np
+    import torch
+    N, T = batch.num_envs, out["reward"].shape[0]
+    per_env = (T * (batch.obs_dim * out["obs"].element_size() + out["reward"].element_size() + 4)
+               + batch.state.shape[0] * batch.state.element_size())
+    k = min(N, budget // per_env)
+    ix = torch.as_tensor(np.sort(np.random.default_rng(0).choice(N, k, replace=False)), device=batch.device)
+    return {"obs": out["obs"].index_select(2, ix).cpu().numpy(),
+            "reward": out["reward"].index_select(1, ix).cpu().numpy(),
+            "done": out["done"].index_select(1, ix).float().cpu().numpy(),
+            "state": batch.state.index_select(1, ix).cpu().numpy()}
 
 
 # ---------------------------------------------------------------- clocks sampler
@@ -273,6 +303,8 @@ def run_b200(args):
         barrier()
         l1 = batch.launch_count
         m1 = clk.mark()
+        # what the last timed step computed, before the passes below overwrite `out` and advance the envs
+        dumped = sample_outputs(batch, out, DUMP_BYTES // world) if args.dump_outputs else None
         # kernel-only duration of the dominant kernel (rollout launches back to back, same stream)
         k0, k1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         k0.record()
@@ -288,6 +320,11 @@ def run_b200(args):
                 batch.rollout(T, actions, out=out)
             torch.cuda.synchronize(dev)
         m2 = clk.mark()
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        sfx = f"_rank{rank}" if world > 1 else ""
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}{sfx}.npy"), a)
     kern_ms = k0.elapsed_time(k1) / args.steps
     clocks = clk.summary(m0, max(m2, m0 + 1))
     clocks["samples_in_timed_region"] = m1 - m0

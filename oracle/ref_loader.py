@@ -1,16 +1,17 @@
 """TEST INFRASTRUCTURE ONLY -- loads the *unmodified* reference env files.
 
-The reference (``/root/reference``) is pure Python but imports ``gym`` / ``gymnasium`` /
+The reference (a checkout of gym-lorenz named by ``GYM_LORENZ_REFERENCE``) is pure Python but imports ``gym`` / ``gymnasium`` /
 ``stable_baselines3`` / ``matplotlib`` at module top, none of which is installed in this
 image.  The env classes only use ``gym.Env`` as a base class, ``spaces.Box`` and (PMSM)
 ``Env.reset(seed) -> self.np_random``.  This module injects minimal stub modules into
 ``sys.modules`` and then executes the reference files *by path*, unchanged, so the
 arithmetic that runs is the reference's own.
 
-It works only where ``/root/reference`` exists (the build container).  It is used by
+The reference is not part of this repository: this module works only where
+``GYM_LORENZ_REFERENCE`` points at a checkout of it.  It is used by
 ``tests/golden/make_golden.py`` to generate the committed fixtures and by the CPU test
 suite to pin ``oracle/chaos_oracle.c``.  Nothing in the product package imports it, and
-nothing that runs on the GPU box depends on it.
+nothing on the GPU side of the suite depends on it.
 """
 from __future__ import annotations
 
@@ -21,12 +22,12 @@ import types
 
 import numpy as np
 
-REF_ROOT = os.environ.get("GYM_LORENZ_REFERENCE", "/root/reference")
+REF_ROOT = os.environ.get("GYM_LORENZ_REFERENCE", "")
 ENV_DIR = os.path.join(REF_ROOT, "code", "gym-lorenz", "gym_lorenz", "envs")
 
 
 def available() -> bool:
-    return os.path.isdir(ENV_DIR)
+    return bool(REF_ROOT) and os.path.isdir(ENV_DIR)
 
 
 class _Box:

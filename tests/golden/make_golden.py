@@ -1,10 +1,10 @@
-"""Generates the committed golden vectors from the UNMODIFIED reference (container-only).
+"""Generates the committed golden vectors from the UNMODIFIED reference (needs its sources).
 
-    python tests/golden/make_golden.py        # needs /root/reference
+    GYM_LORENZ_REFERENCE=<gym-lorenz checkout> python tests/golden/make_golden.py
 
 Outputs (tests/golden/*.npz) -- all produced by executing the reference's own env classes
 through oracle/ref_loader.py, or read from the reference's own artefact
-/root/reference/PMSM_Origin_Data.xlsx (written by code/lorenz_pmsm/test_evaluate.py:61-166):
+$GYM_LORENZ_REFERENCE/PMSM_Origin_Data.xlsx (written by code/lorenz_pmsm/test_evaluate.py:61-166):
 
   cfg1_lorenz3.npz    BASELINE.json configs[0]: dynamic.py::lorenzEnv_transient, N=1,
                       np.random.seed(0); reset(); 1000 steps with

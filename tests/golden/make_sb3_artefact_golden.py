@@ -1,6 +1,6 @@
-"""Extracts what the reference's own SB3 artefacts hold about the wrappers around the env (container-only).
+"""Extracts what the reference's own SB3 artefacts hold about the wrappers around the env (needs its sources).
 
-    python tests/golden/make_sb3_artefact_golden.py        # needs /root/reference
+    GYM_LORENZ_REFERENCE=<gym-lorenz checkout> python tests/golden/make_sb3_artefact_golden.py
 
 The reference ships eight finished training runs of code/lorenz_pmsm/train.py:152-190
 (`DummyVecEnv([Monitor(make_env(alpha))])` -> `VecNormalize(norm_obs=True, norm_reward=False,
@@ -31,7 +31,7 @@ import zipfile
 
 import numpy as np
 
-REF = "/root/reference"
+REF = os.environ["GYM_LORENZ_REFERENCE"]
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 

@@ -3,8 +3,8 @@ is attempted without a GPU, and the product fails loudly instead of falling back
 import ctypes as C
 import os
 import re
-
-import pytest
+import subprocess
+import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -67,13 +67,19 @@ def test_create_validates_arguments(chaos_lib):
 
 
 def test_no_cpu_fallback_without_gpu():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from gym_lorenz_b200 import ChaosLibError
-    from gym_lorenz_b200.vec_env import BatchedChaosVecEnv
-    with pytest.raises(ChaosLibError):
-        BatchedChaosVecEnv("hr_sync", 4)
+    """Runs in a child process that sees no GPU (CUDA_VISIBLE_DEVICES empty), so it also runs where a GPU is present."""
+    code = ("import sys\n"
+            f"sys.path.insert(0, {ROOT!r})\n"
+            "from gym_lorenz_b200 import ChaosLibError\n"
+            "from gym_lorenz_b200.vec_env import BatchedChaosVecEnv\n"
+            "try:\n"
+            "    BatchedChaosVecEnv('hr_sync', 4)\n"
+            "except ChaosLibError as e:\n"
+            "    print('raised:', e)\n")
+    r = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert r.stdout.startswith("raised:"), r.stdout
 
 
 def test_product_never_imports_the_oracle():

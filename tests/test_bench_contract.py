@@ -6,6 +6,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BASE_KEYS = {"metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better",
              "scaling", "vs_baseline", "dtype", "data", "config", "e2e", "cpu_baseline", "gpu_launches"}
@@ -60,3 +63,32 @@ def test_committed_b200_line_has_the_contract_keys():
     assert not ({"hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown"} & set(c["reasons"]))
     assert d["e2e"]["h2d_bytes_per_step"] > 0 and d["e2e"]["d2h_bytes_per_step"] > 0
     assert d["e2e"]["value"] < d["value"]          # the host-buffer path cannot repeat the device-timed number
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_repeatable_and_follow_steps(tmp_path):
+    """--dump-outputs at the bench shape: float32/float64 arrays of at most 64 MB in all, identical for identical
+    arguments.  Every warm-up and timed step is one rollout of the same envs, so the last timed step of 4 warm-up + 3
+    timed steps computes what that of 3 + 4 does: equal dumps pin both --steps and the moment the dump is taken."""
+    def run(warmup, steps, d):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", str(warmup),
+                              "--no-e2e", "--no-cpu-baseline", "--dump-outputs", str(d)],
+                             capture_output=True, text=True, timeout=600, check=True).stdout.strip().splitlines()
+        line = json.loads(out[-1])
+        assert line["steps"] == line["gpu_launches"] == steps and line["warmup"] == warmup
+        assert sum(f.stat().st_size for f in d.iterdir()) <= 64_000_000
+        return {f.stem: np.load(f) for f in d.iterdir() if f.suffix == ".npy"}
+
+    a, b, c = run(4, 3, tmp_path / "a"), run(4, 3, tmp_path / "b"), run(3, 4, tmp_path / "c")
+    assert sorted(a) == ["done", "obs", "reward", "state"]
+    assert all(x.dtype in (np.float32, np.float64) for x in a.values())
+    T, k = a["reward"].shape
+    assert T == 256 and 0 < k <= 65536 and a["obs"].shape == (T, 6, k) and a["state"].shape[1] == k
+    assert np.isin(a["done"], (0, 1, 2, 3)).all()
+    # the state is the one the dumped step left: its last observation holds the positions (f32) of that state
+    live = a["done"][-1] == 0
+    assert live.any()
+    assert np.array_equal(a["obs"][-1, :3, live], a["state"][:3, live].astype(np.float32).T, equal_nan=True)
+    for name in a:
+        assert np.array_equal(a[name], b[name], equal_nan=True), name
+        assert np.array_equal(a[name], c[name], equal_nan=True), name
