@@ -82,6 +82,19 @@ class RolloutDesc(C.Structure):
     ]
 
 
+POLICY_HIDDEN = 64   # CL_POLICY_HIDDEN
+
+
+class Policy(C.Structure):
+    _fields_ = [
+        ("params", C.c_void_p), ("obs_mean", C.c_void_p), ("obs_var", C.c_void_p),
+        ("epsilon", C.c_double), ("clip_obs", C.c_double),
+        ("obs0", C.c_void_p), ("obs0_es", C.c_int64), ("obs0_cs", C.c_int64),
+        ("obs_last", C.c_void_p), ("act_out", C.c_void_p), ("metrics", C.c_void_p),
+        ("steady_start", C.c_int32), ("dt", C.c_double), ("error_band", C.c_double),
+    ]
+
+
 class HostView(C.Structure):
     _fields_ = [
         ("obs", C.c_void_p), ("reward", C.c_void_p), ("done", C.c_void_p),
@@ -102,6 +115,8 @@ SYMBOLS = [
     ("cl_init_persistent", C.c_int, [_VP, _VP, C.POINTER(Buffers)]),
     ("cl_step", C.c_int, [_VP, _VP, C.POINTER(Buffers), C.POINTER(IO)]),
     ("cl_rollout", C.c_int, [_VP, _VP, C.POINTER(Buffers), C.POINTER(IO), C.POINTER(RolloutDesc)]),
+    ("cl_policy_rollout", C.c_int, [_VP, _VP, C.POINTER(Buffers), C.POINTER(IO), C.POINTER(RolloutDesc),
+                                    C.POINTER(Policy)]),
     ("cl_derivatives", C.c_int, [_VP, _VP, _VP, _VP, _VP, C.c_int64]),
     ("cl_stats", C.c_int, [_VP, _VP, C.POINTER(Buffers), _VP, C.c_int]),
     ("cl_get_step_index", C.c_int, [_VP, C.POINTER(C.c_uint64)]),

@@ -1,8 +1,10 @@
 """In-tree build of libchaos_b200.so for sm_100a (nvcc cross-compiles without a GPU).
 
-Two translation units carry kernels:
+The kernels live in four translation units:
   * tu_parity.cu     -fmad=false : parity env kinds, IEEE two-rounding arithmetic
   * tu_northstar.cu  (fmad on)   : RK4 x S kinds + FMA-peak micro-kernel
+  * tu_rl_ops.cu     -fmad=false : SB3 plumbing around the step (GAE, VecNormalize, metrics, ...)
+  * tu_policy.cu     -fmad=false : MlpPolicy fused into the hr_sync / pmsm_sync rollout
 plus chaos_b200.cu, the C-ABI host side.  The CUDA runtime is linked statically so the
 library does not depend on which libcudart PyTorch bundles.
 """
@@ -51,6 +53,7 @@ def build_library(force: bool = False, verbose: bool = False) -> str:
         ("tu_parity.cu", ["-fmad=false"]),
         ("tu_northstar.cu", []),
         ("tu_rl_ops.cu", ["-fmad=false"]),
+        ("tu_policy.cu", ["-fmad=false"]),
         ("chaos_b200.cu", []),
     ]
     def compile_unit(unit):
@@ -63,7 +66,7 @@ def build_library(force: bool = False, verbose: bool = False) -> str:
         subprocess.run(cmd, check=True)
         return obj
 
-    # the four translation units are independent: compile them side by side (55 s -> the longest unit)
+    # the translation units are independent: compile them side by side (55 s -> the longest unit)
     with ThreadPoolExecutor(max_workers=len(units)) as pool:
         objs = list(pool.map(compile_unit, units))
     cmd = [nvcc, *ARCH, "-shared", "-cudart", "static", "-o", LIB, *objs]

@@ -312,6 +312,15 @@ __global__ void k_relay(const uint32_t* host_words, uint32_t* dev_words, uint32_
   cl::relay_lanes(host_words, dev_words, gen, lanes, spl, nslices, host_err);
 }
 
+// graph mode: the device-resident Philox step index (CUDA graphs) advances after each env kernel
+static int advance_graph_step(cl_ctx* ctx, cudaStream_t st, uint64_t count) {
+  if (!ctx->graph_mode) return CL_OK;
+  k_advance_step<<<1, 1, 0, st>>>(ctx->d_step, count);
+  const cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return fail(ctx, CL_ECUDA, "step-index advance failed: %s", cudaGetErrorString(e));
+  return CL_OK;
+}
+
 static int launch(cl_ctx* ctx, const KParams& p_in, int mode, cudaStream_t st) {
   KParams p = p_in;
   int32_t plain = 0;
@@ -322,13 +331,8 @@ static int launch(cl_ctx* ctx, const KParams& p_in, int mode, cudaStream_t st) {
   ctx->launches += 1;
   ctx->plain_launches += (plain & 1);
   ctx->sm_launches += (plain >> 1) & 1;
-  if (ctx->graph_mode && mode != cl::MODE_INIT) {  // device-resident Philox step index (CUDA graphs)
-    const uint64_t count = (mode == cl::MODE_ROLLOUT || mode == cl::MODE_ROLLOUT_DYN) ? (uint64_t)p.T : 1;
-    k_advance_step<<<1, 1, 0, st>>>(ctx->d_step, count);
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(ctx, CL_ECUDA, "step-index advance failed: %s", cudaGetErrorString(e));
-  }
-  return CL_OK;
+  if (mode == cl::MODE_INIT) return CL_OK;
+  return advance_graph_step(ctx, st, (mode == cl::MODE_ROLLOUT || mode == cl::MODE_ROLLOUT_DYN) ? (uint64_t)p.T : 1);
 }
 
 extern "C" int cl_init_persistent(cl_ctx* ctx, void* stream, const cl_buffers* buf) {
@@ -489,6 +493,35 @@ extern "C" int cl_rollout(cl_ctx* ctx, void* stream, const cl_buffers* buf, cons
     }
   }
   r = launch(ctx, p, mode, st);
+  if (r == CL_OK) ctx->step_index += (uint64_t)d->T;
+  return r;
+}
+
+extern "C" int cl_policy_rollout(cl_ctx* ctx, void* stream, const cl_buffers* buf, const cl_io* io,
+                                 const cl_rollout_desc* d, const cl_policy* pol) {
+  if (!ctx) return fail(nullptr, CL_EINVAL, "null ctx");
+  const int kind = ctx->cfg.kind;
+  if (kind != CL_ENV_HR_SYNC && kind != CL_ENV_PMSM_SYNC)
+    return fail(ctx, CL_EINVAL, "cl_policy_rollout: env kind %d is not supported (hr_sync and pmsm_sync only)", kind);
+  if (ctx->cfg.flags & CL_F_OBS_F64) return fail(ctx, CL_EINVAL, "cl_policy_rollout: float32 observations only");
+  if (!io || !d || !pol || d->T < 1) return fail(ctx, CL_EINVAL, "cl_policy_rollout: io/desc/policy required, T >= 1");
+  if (io->action || io->noise) return fail(ctx, CL_EINVAL, "cl_policy_rollout: io.action and io.noise must be NULL");
+  if (!pol->params || !pol->obs0) return fail(ctx, CL_EINVAL, "cl_policy_rollout: params and obs0 are required");
+  if ((pol->obs_mean == nullptr) != (pol->obs_var == nullptr))
+    return fail(ctx, CL_EINVAL, "cl_policy_rollout: obs_mean and obs_var go together");
+  if (pol->steady_start < 0 || pol->steady_start >= d->T)
+    return fail(ctx, CL_EINVAL, "cl_policy_rollout: steady_start %d outside [0, T)", pol->steady_start);
+  KParams p;
+  int r = fill_params(ctx, buf, io, p);
+  if (r) return r;
+  p.T = d->T; p.obs_ts = d->obs_ts; p.rew_ts = d->rew_ts; p.done_ts = d->done_ts;
+  cudaStream_t st = (cudaStream_t)stream;
+  CU(cudaSetDevice(ctx->cfg.device));
+  const cudaError_t e = cl_launch_policy(kind, p, *pol, (float)ctx->lay.act_low, (float)ctx->lay.act_high, st,
+                                         ctx->sm_count);
+  if (e != cudaSuccess) return fail(ctx, CL_ECUDA, "policy rollout launch failed: %s", cudaGetErrorString(e));
+  ctx->launches += 1;
+  r = advance_graph_step(ctx, st, (uint64_t)d->T);
   if (r == CL_OK) ctx->step_index += (uint64_t)d->T;
   return r;
 }

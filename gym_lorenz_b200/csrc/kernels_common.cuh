@@ -346,7 +346,8 @@ __device__ __forceinline__ unsigned env_interval(typename E::S& s, int32_t& ep_l
                                              const unsigned lane, const int t, const uint64_t step,
                                              const float* a, const bool want_noise, const bool obs64,
                                              const bool autoreset, unsigned& bad_acc, float* sm_rows, bool& fin,
-                                             PlainPending<E>* pend = nullptr, double* blk_stats = nullptr) {
+                                             PlainPending<E>* pend = nullptr, double* blk_stats = nullptr,
+                                             typename E::real* obs_out = nullptr) {
   typedef typename E::real real;
   if (PLAIN && CL_PLAIN_DEFER) plain_emit<E, RUNPTR>(p, i, live, *pend);   // outputs of the previous interval
   // The per-interval Philox stream (key / counter words).  Generic kernels build it up front: building
@@ -473,6 +474,12 @@ __device__ __forceinline__ unsigned env_interval(typename E::S& s, int32_t& ep_l
     pend->dflags = (uint32_t)((term ? CL_DONE_TERMINATED : 0) | (trunc ? CL_DONE_TRUNCATED : 0));
     pend->t = t;
     pend->valid = 1u;
+  }
+  // the observation the env is in now (the reset observation where it auto-reset): the policy rollout's
+  // next input.  Every other caller leaves obs_out null and the copy compiles away.
+  if (obs_out != nullptr) {
+#pragma unroll
+    for (int c = 0; c < E::OBS; ++c) obs_out[c] = obs[c];
   }
   return dall;
 }
@@ -1300,4 +1307,7 @@ cudaError_t cl_occupancy_parity(int kind, int block, int* blocks_per_sm);
 cudaError_t cl_occupancy_northstar(int kind, int block, int* blocks_per_sm);
 cudaError_t cl_dyn_occupancy_parity(int kind, int chunk, int* blocks_per_sm);
 cudaError_t cl_dyn_occupancy_northstar(int kind, int chunk, int* blocks_per_sm);
+// tu_policy.cu
+cudaError_t cl_launch_policy(int kind, const cl::KParams& p, const cl_policy& q, float act_lo, float act_hi,
+                             cudaStream_t st, int sms);
 cudaError_t cl_fma_peak_launch(int dtype_bytes, int grid, int block, int iters, void* sink, cudaStream_t st);

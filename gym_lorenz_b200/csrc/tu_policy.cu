@@ -1,0 +1,230 @@
+// Translation unit of cl_policy_rollout: a trained SB3 MlpPolicy (deterministic actions) fused into the
+// hr_sync / pmsm_sync rollout, with the evaluation metrics of cl_eval_metrics accumulated on the fly.
+// Built with -fmad=false (see build.py), like tu_parity.cu, so the env arithmetic is bit-identical to
+// cl_rollout's; every fused operation of the policy is an explicit fmaf.
+#include "envs_parity.cuh"
+
+using namespace cl;
+
+// Weight placement (A/B in DESIGN.md section 11c): 0 = staged once per block in shared memory and read
+// with warp-uniform broadcast loads; 1 = a __grid_constant__ kernel parameter (constant-bank operands),
+// which needs the weights on the host: the launch then copies them back and synchronises the stream.
+#ifndef CL_POLICY_W_PARAM
+#define CL_POLICY_W_PARAM 0
+#endif
+
+namespace {
+
+constexpr int H = CL_POLICY_HIDDEN;
+
+// cl_policy.params, torch Linear layout: W1[H][OBS] b1[H] W2[H][H] b2[H] W3[ACT][H] b3[ACT]
+template <int OBS, int ACT>
+struct PolicyLayout {
+  enum {
+    W1 = 0, B1 = W1 + H * OBS, W2 = B1 + H, B2 = W2 + H * H, W3 = B2 + H, B3 = W3 + ACT * H,
+    TOTAL = B3 + ACT, PADDED = (TOTAL + 3) & ~3
+  };
+  static_assert(W2 % 4 == 0, "W2 rows are read as float4");
+};
+
+template <class E, bool PARAM> struct WeightArg { struct type { float unused; }; };
+template <class E> struct WeightArg<E, true> {
+  struct type { float w[PolicyLayout<E::OBS, E::ACT>::PADDED]; };
+};
+
+// One thread per env for the whole launch (the MLP costs the same for every env: no task queue).
+// Per control interval: frozen VecNormalize -> MLP (float32, fixed fmaf order) -> clip to the action box
+// -> the same env_interval<E, ROLL> cl_rollout runs, with the same Philox step index -> metrics in f64.
+template <class E, bool PARAM>
+__global__ void __launch_bounds__(128, 4) k_policy_rollout(const KParams p, const cl_policy q, const float lo,
+                                                           const float hi,
+                                                           const __grid_constant__ typename WeightArg<E, PARAM>::type wp) {
+  typedef typename E::real real;
+  constexpr int OBS = E::OBS, ACT = E::ACT, NERR = 3;
+  typedef PolicyLayout<OBS, ACT> LW;
+  __shared__ __align__(16) float s_w[PARAM ? 4 : LW::PADDED];
+  __shared__ double s_mean[OBS], s_sd[OBS];
+  const float* W;
+  if constexpr (PARAM) {
+    W = wp.w;
+  } else {
+    for (int k = threadIdx.x; k < LW::TOTAL; k += blockDim.x) s_w[k] = q.params[k];
+    W = s_w;
+  }
+  const bool norm = q.obs_mean != nullptr;
+  if (norm && threadIdx.x < OBS) {
+    // k_normalize's expression: the division stays a division by sqrt(var + eps)
+    s_mean[threadIdx.x] = q.obs_mean[threadIdx.x];
+    s_sd[threadIdx.x] = sqrt(q.obs_var[threadIdx.x] + q.epsilon);
+  }
+  __syncthreads();
+
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const bool live = i < p.n;
+  const unsigned lane = threadIdx.x & 31u;
+  typename E::S s = {};
+  int32_t ep_len = 0;
+  double ep_ret = 0.0;
+  float ob[OBS];
+#pragma unroll
+  for (int c = 0; c < OBS; ++c) ob[c] = 0.0f;
+  if (live) {
+    E::load(s, p, i);
+    ep_len = p.ep_len[i];
+    ep_ret = p.ep_return[i];
+#pragma unroll
+    for (int c = 0; c < OBS; ++c) ob[c] = q.obs0[i * q.obs0_es + c * q.obs0_cs];
+  }
+  E::prepare(s, p, live);
+  const bool autoreset = (p.flags & CL_F_AUTORESET) != 0;
+  const bool want_noise = E::NOISE > 0 && E::uses_noise(p);
+  const float4* W2v = reinterpret_cast<const float4*>(W + LW::W2);
+
+  // metrics (cl_eval_metrics): sum |e_c| and e_c^2 over t >= steady_start, last t with |e_c| > band, sum |u|^2
+  double sa[NERR], sq[NERR], en = 0.0;
+  int last_ex[NERR];
+#pragma unroll
+  for (int c = 0; c < NERR; ++c) { sa[c] = 0.0; sq[c] = 0.0; last_ex[c] = -1; }
+
+  unsigned bad_acc = 0u;
+  bool fin = E::finite(s);
+  const uint64_t step0 = step_base(p);
+  for (int t = 0; t < p.T; ++t) {
+    float z[OBS];
+#pragma unroll
+    for (int c = 0; c < OBS; ++c) {
+      if (norm) {
+        double v = ((double)ob[c] - s_mean[c]) / s_sd[c];
+        v = v < -q.clip_obs ? -q.clip_obs : (v > q.clip_obs ? q.clip_obs : v);
+        z[c] = (float)v;
+      } else {
+        z[c] = ob[c];
+      }
+    }
+    // h1 stays in registers; h2 is produced four units at a time (four independent FMA chains) and folded
+    // straight into the action accumulators, so it is never stored
+    float h1[H];
+#pragma unroll
+    for (int j = 0; j < H; ++j) {
+      float acc = W[LW::B1 + j];
+#pragma unroll
+      for (int c = 0; c < OBS; ++c) acc = fmaf(W[LW::W1 + j * OBS + c], z[c], acc);
+      h1[j] = tanhf(acc);
+    }
+    float a[ACT];
+#pragma unroll
+    for (int c = 0; c < ACT; ++c) a[c] = W[LW::B3 + c];
+#pragma unroll 1
+    for (int j = 0; j < H; j += 4) {
+      float acc[4];
+#pragma unroll
+      for (int u = 0; u < 4; ++u) acc[u] = W[LW::B2 + j + u];
+#pragma unroll
+      for (int k4 = 0; k4 < H / 4; ++k4) {
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+          const float4 w = W2v[(j + u) * (H / 4) + k4];
+          acc[u] = fmaf(w.x, h1[4 * k4 + 0], acc[u]);
+          acc[u] = fmaf(w.y, h1[4 * k4 + 1], acc[u]);
+          acc[u] = fmaf(w.z, h1[4 * k4 + 2], acc[u]);
+          acc[u] = fmaf(w.w, h1[4 * k4 + 3], acc[u]);
+        }
+      }
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        const float h2 = tanhf(acc[u]);
+#pragma unroll
+        for (int c = 0; c < ACT; ++c) a[c] = fmaf(W[LW::W3 + c * H + j + u], h2, a[c]);
+      }
+    }
+#pragma unroll
+    for (int c = 0; c < ACT; ++c) a[c] = clipf(a[c], lo, hi);   // SB3 predict: np.clip to the Box
+    if (q.act_out != nullptr && live) {
+#pragma unroll
+      for (int c = 0; c < ACT; ++c) q.act_out[((int64_t)t * p.n + i) * ACT + c] = a[c];
+    }
+    real nob[OBS];
+    env_interval<E, true>(s, ep_len, ep_ret, p, i, live, lane, t, step0 + (uint64_t)t, a, want_noise, false,
+                          autoreset, bad_acc, nullptr, fin, nullptr, nullptr, nob);
+#pragma unroll
+    for (int c = 0; c < OBS; ++c) ob[c] = (float)nob[c];
+#pragma unroll
+    for (int c = 0; c < NERR; ++c) {
+      const double e = (double)ob[c];
+      if (fabs(e) > q.error_band) last_ex[c] = t;
+      if (t >= q.steady_start) { sa[c] += fabs(e); sq[c] += e * e; }
+    }
+    double u2 = 0.0;
+#pragma unroll
+    for (int c = 0; c < ACT; ++c) u2 += (double)a[c] * (double)a[c];
+    en += u2;
+  }
+  if (bad_acc && lane == 0) atomicAdd(&p.stats[CL_STAT_NONFINITE], (double)bad_acc);
+  if (!live) return;
+  E::store(s, p, i);
+  p.ep_len[i] = ep_len;
+  p.ep_return[i] = ep_ret;
+  if (q.obs_last != nullptr) {
+#pragma unroll
+    for (int c = 0; c < OBS; ++c) q.obs_last[i * q.obs0_es + c * q.obs0_cs] = ob[c];
+  }
+  if (q.metrics != nullptr) {
+    // k_eval_final's combination: averages over components, settling time as np.nanmax over components
+    const double m = (double)(p.T - q.steady_start);
+    double mae = 0.0, rmse = 0.0, ts = -1.0;
+    bool never = false;
+#pragma unroll
+    for (int c = 0; c < NERR; ++c) {
+      mae += sa[c] / m;
+      rmse += sqrt(sq[c] / m);
+      if (last_ex[c] + 1 >= p.T) never = true;
+      const double tc = (last_ex[c] < 0) ? 0.0 : (double)(last_ex[c] + 1) * q.dt;
+      if (last_ex[c] + 1 < p.T && tc > ts) ts = tc;
+    }
+    double* o = q.metrics + i * 4;
+    o[0] = mae / NERR;
+    o[1] = rmse / NERR;
+    o[2] = (ts < 0.0 && never) ? nan("") : (ts < 0.0 ? 0.0 : ts);
+    o[3] = en * q.dt;
+  }
+}
+
+// Threads of the fullest SM decide the launch: ceil(blocks / SMs) * block, ties -> the larger block (a
+// smaller one stages the weights into shared memory more often: 14 blocks of 32 would not fit one SM).
+int policy_block(int64_t n, int sms) {
+  int best = 128;
+  int64_t best_cost = -1;
+  for (int b = 128; b >= 32; b /= 2) {
+    const int64_t cost = (((n + b - 1) / b + sms - 1) / sms) * b;
+    if (best_cost < 0 || cost < best_cost) { best_cost = cost; best = b; }
+  }
+  return best;
+}
+
+template <class E>
+cudaError_t launch_policy(const KParams& p, const cl_policy& q, float lo, float hi, cudaStream_t st, int sms) {
+  typedef PolicyLayout<E::OBS, E::ACT> LW;
+  const int block = policy_block(p.n, sms);
+  const unsigned grid = (unsigned)((p.n + block - 1) / block);
+  typename WeightArg<E, CL_POLICY_W_PARAM != 0>::type w;
+  memset(&w, 0, sizeof(w));
+#if CL_POLICY_W_PARAM
+  cudaError_t e = cudaMemcpyAsync(w.w, q.params, sizeof(float) * LW::TOTAL, cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  if (e != cudaSuccess) return e;
+#endif
+  (void)sizeof(LW);
+  k_policy_rollout<E, CL_POLICY_W_PARAM != 0><<<grid, block, 0, st>>>(p, q, lo, hi, w);
+  return cudaGetLastError();
+}
+
+}  // namespace
+
+cudaError_t cl_launch_policy(int kind, const KParams& p, const cl_policy& q, float lo, float hi, cudaStream_t st,
+                             int sms) {
+  switch (kind) {
+    case CL_ENV_HR_SYNC: return launch_policy<EnvHRSync>(p, q, lo, hi, st, sms);
+    case CL_ENV_PMSM_SYNC: return launch_policy<EnvPMSMSync>(p, q, lo, hi, st, sms);
+    default: return cudaErrorInvalidValue;
+  }
+}

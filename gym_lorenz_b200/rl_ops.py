@@ -6,16 +6,21 @@ in csrc/tu_rl_ops.cu.
   DeviceVecNormalize     SB3 VecNormalize(norm_obs, norm_reward, clip_obs) (code/lorenz_pmsm/train.py:118,170)
   DeviceVecFrameStack    SB3 VecFrameStack(n_stack)                        (code/lorenz_filter/train.py:115)
   eval_metrics(...)      calculate_advanced_metrics + steady-state MAE/RMSE (code/lorenz_pmsm/test_evaluate.py:25-59,239-250)
+  evaluate_policy(...)   the predict loop of those scripts + eval_metrics, one launch (csrc/tu_policy.cu)
   DeviceRolloutCollector SB3 OnPolicyAlgorithm.collect_rollouts without NumPy / host round trips
 """
 from __future__ import annotations
 
 import ctypes as C
+import os
+import zipfile
+from io import BytesIO
 from typing import Callable, Dict, Optional, Tuple
 
 import torch
 
 from . import _lib as L
+from .core import ChaosBatch
 
 
 def _p(t: Optional[torch.Tensor]):
@@ -64,6 +69,152 @@ def eval_metrics(err: torch.Tensor, ctrl: torch.Tensor, dt: float, error_band: f
         L.check(lib.cl_eval_metrics(_stream(dev), _p(err), _p(ctrl), T, ne, nc, N, N, int(steady_start), float(dt),
                                     float(error_band), _p(out)), None, "cl_eval_metrics")
     return {"mae": out[:, 0], "rmse": out[:, 1], "settling_time": out[:, 2], "energy": out[:, 3]}
+
+
+# kinds cl_policy_rollout serves (the reference trains policies on these two) -> control interval (s)
+_POLICY_DT = {L.HR_SYNC: 0.001, L.PMSM_SYNC: 0.001}
+_SB3_KEYS = ("mlp_extractor.policy_net.0.weight", "mlp_extractor.policy_net.0.bias",
+             "mlp_extractor.policy_net.2.weight", "mlp_extractor.policy_net.2.bias",
+             "action_net.weight", "action_net.bias")
+_RECORDABLE = ("obs", "action", "reward", "done")
+
+
+def _policy_kind(kind) -> int:
+    k = L.KIND_NAMES.get(kind, -1) if isinstance(kind, str) else int(kind)
+    if k not in _POLICY_DT:
+        raise ValueError(f"policy evaluation supports hr_sync and pmsm_sync only, got {kind!r}")
+    return k
+
+
+def pack_policy(src, device, kind="hr_sync") -> torch.Tensor:
+    """The float32 parameter block `cl_policy_rollout` reads, in torch Linear layout:
+    W1[64][obs_dim] b1[64] W2[64][64] b2[64] W3[act_dim][64] b3[act_dim].
+
+    `src` is one of
+      * a stable-baselines3 `ActorCriticPolicy` state dict (`mlp_extractor.policy_net.{0,2}.{weight,bias}`,
+        `action_net.{weight,bias}`; the value head and `log_std` are ignored);
+      * the path of an SB3 model zip: its `policy.pth` member is read with `zipfile` and
+        `torch.load(weights_only=True)`, SB3 itself is not needed.  The key names follow SB3 2.7.1's
+        source; they have not been checked against the reference's own saved models;
+      * a `(policy_net, action_net)` pair of torch modules: Linear-Tanh-Linear-Tanh and a Linear.
+
+    Every shape is checked against `kind`'s observation / action dimensions and the [64, 64] MlpPolicy
+    architecture; a mismatch raises ValueError before anything reaches the device.
+    """
+    k = _policy_kind(kind)
+    lay = L.layout(k)
+    obs_dim, act_dim, h = lay.obs_dim, lay.act_dim, L.POLICY_HIDDEN
+    if isinstance(src, (str, os.PathLike)):
+        with zipfile.ZipFile(src) as z:
+            if "policy.pth" not in z.namelist():
+                raise ValueError(f"{src}: no policy.pth member (not an SB3 model zip)")
+            src = torch.load(BytesIO(z.read("policy.pth")), map_location="cpu", weights_only=True)
+    if isinstance(src, (tuple, list)):
+        if len(src) != 2 or not all(isinstance(m, torch.nn.Module) for m in src):
+            raise ValueError("expected a (policy_net, action_net) pair of torch modules")
+        pnet, anet = src
+        leaves = [m for m in pnet.modules() if len(list(m.children())) == 0]
+        if [type(m) for m in leaves] != [torch.nn.Linear, torch.nn.Tanh, torch.nn.Linear, torch.nn.Tanh] or \
+                not isinstance(anet, torch.nn.Linear):
+            raise ValueError("policy_net must be Linear-Tanh-Linear-Tanh and action_net a Linear "
+                             "(SB3 MlpPolicy, pi=[64, 64], activation_fn=Tanh)")
+        tensors = [leaves[0].weight, leaves[0].bias, leaves[2].weight, leaves[2].bias, anet.weight, anet.bias]
+    elif isinstance(src, dict):
+        missing = [key for key in _SB3_KEYS if key not in src]
+        if missing:
+            raise ValueError(f"not an SB3 MlpPolicy state dict: missing {missing}")
+        extra = sorted(key for key in src if key.startswith("mlp_extractor.policy_net.") and key not in _SB3_KEYS)
+        if extra:
+            raise ValueError(f"policy_net is not [64, 64]: unexpected {extra}")
+        tensors = [src[key] for key in _SB3_KEYS]
+    else:
+        raise ValueError(f"cannot pack a policy from {type(src).__name__}")
+    shapes = [(h, obs_dim), (h,), (h, h), (h,), (act_dim, h), (act_dim,)]
+    for key, t, shape in zip(_SB3_KEYS, tensors, shapes):
+        if t is None or tuple(t.shape) != shape:
+            got = None if t is None else tuple(t.shape)
+            raise ValueError(f"{key}: expected shape {shape}, got {got}")
+    with torch.no_grad():
+        return torch.cat([t.detach().reshape(-1).to(torch.float32).cpu() for t in tensors]).to(device)
+
+
+def evaluate_policy(env, policy, T: int, *, normalize=None, dt: Optional[float] = None, error_band: float = 0.05,
+                    steady_start: Optional[int] = None, record=(), obs0: Optional[torch.Tensor] = None
+                    ) -> Dict[str, torch.Tensor]:
+    """Roll a trained policy deterministically for T control intervals in ONE launch and return the
+    evaluation metrics of `eval_metrics` without storing the trajectories: the reference's
+    `model.predict(obs, deterministic=True)` loops (code/test_evaluate.py, code/lorenz_pmsm/test_evaluate.py).
+
+    env: a BatchedChaosVecEnv (or device wrapper around one) or a ChaosBatch of kind hr_sync / pmsm_sync.
+    policy: what `pack_policy` accepts, or its packed tensor.  normalize: a DeviceVecNormalize whose
+    `obs_rms`, `epsilon` and `clip_obs` are used frozen, or None.  dt defaults to the control interval,
+    steady_start to min(1000, T // 2).  obs0 (f32 [N, obs_dim]) is the observation interval 0 acts on;
+    by default the batch's observation planes, which hold it after `reset()` / `step()` -- after
+    `set_attr(...)` or `rollout()` pass it explicitly.  The last observation is written back to the
+    observation planes, so a following `step()` or `evaluate_policy` continues from there.
+
+    Returns {"mae", "rmse", "settling_time", "energy"} (f64 [N] device tensors) plus the streams named in
+    `record`: "obs" f32 [T, obs_dim, n_pad], "reward" [T, n_pad], "done" u8 [T, n_pad] (as `rollout`) and
+    "action" f32 [T, N, act_dim] (the clipped actions applied).
+
+    For an evaluation like the reference's use a ChaosBatch(autoreset=False) with max_episode_steps >= T:
+    with auto-reset on, the window contains the reset observations, as the recorded streams show.
+    The metrics are in observation units.  For hr_sync the error components are err / 50 (the env's
+    scale_factor): for state units pass error_band=0.05 / 50 and multiply MAE / RMSE by 50.
+    """
+    b = env if isinstance(env, ChaosBatch) else base_batch(env)
+    kind = _policy_kind(b.kind)
+    if b.obs_f64:
+        raise ValueError("evaluate_policy needs float32 observations (obs_f64=False)")
+    T = int(T)
+    if T < 1:
+        raise ValueError("T must be >= 1")
+    if steady_start is None:
+        steady_start = min(1000, T // 2)          # test_evaluate.py:239, as eval_metrics
+    if not 0 <= int(steady_start) < T:
+        raise ValueError(f"steady_start must lie in [0, {T}), got {steady_start}")
+    unknown = [r for r in record if r not in _RECORDABLE]
+    if unknown:
+        raise ValueError(f"record: unknown streams {unknown}; choose from {_RECORDABLE}")
+    params = policy if isinstance(policy, torch.Tensor) else pack_policy(policy, b.device, kind)
+    npar = L.POLICY_HIDDEN * (b.obs_dim + 1 + L.POLICY_HIDDEN + 1 + b.act_dim) + b.act_dim
+    if params.dtype != torch.float32 or params.device != b.device or params.numel() != npar or \
+            not params.is_contiguous():
+        raise ValueError(f"packed policy must be a contiguous f32 tensor of {npar} values on {b.device}")
+    dev, N, NP = b.device, b.num_envs, b.n_pad
+    planes = b._view(b.obs_planes)
+    if obs0 is not None:
+        if not isinstance(obs0, torch.Tensor) or obs0.dtype != torch.float32 or obs0.device != dev or \
+                tuple(obs0.shape) != (N, b.obs_dim):
+            raise ValueError(f"obs0 must be f32 [{N}, {b.obs_dim}] on {dev}")
+        planes.copy_(obs0)
+    out = {}
+    io = L.IO()
+    desc = L.RolloutDesc(T=T)
+    if "obs" in record:
+        out["obs"] = torch.empty((T, b.obs_dim, NP), dtype=torch.float32, device=dev)
+        io.obs, io.obs_es, io.obs_cs, desc.obs_ts = _p(out["obs"]), 1, NP, b.obs_dim * NP
+    if "reward" in record:
+        out["reward"] = torch.empty((T, NP), dtype=b.real, device=dev)
+        io.reward, desc.rew_ts = _p(out["reward"]), NP
+    if "done" in record:
+        out["done"] = torch.empty((T, NP), dtype=torch.uint8, device=dev)
+        io.done, desc.done_ts = _p(out["done"]), NP
+    if "action" in record:
+        out["action"] = torch.empty((T, N, b.act_dim), dtype=torch.float32, device=dev)
+    io.last_ep_ret, io.last_ep_len = _p(b.last_ep_ret), _p(b.last_ep_len)
+    metrics = torch.empty((N, 4), dtype=torch.float64, device=dev)
+    pol = L.Policy(params=_p(params), obs0=_p(b.obs_planes), obs0_es=1, obs0_cs=NP, obs_last=_p(b.obs_planes),
+                   act_out=_p(out.get("action")), metrics=_p(metrics), steady_start=int(steady_start),
+                   dt=float(_POLICY_DT[kind] if dt is None else dt), error_band=float(error_band))
+    if normalize is not None and normalize.norm_obs:
+        pol.obs_mean, pol.obs_var = _p(normalize.obs_rms.mean), _p(normalize.obs_rms.var)
+        pol.epsilon, pol.clip_obs = float(normalize.epsilon), float(normalize.clip_obs)
+    L.check(b.lib.cl_policy_rollout(b.ctx, b._stream(), C.byref(b._bufs), C.byref(io), C.byref(desc), C.byref(pol)),
+            b.ctx, "cl_policy_rollout")
+    b._keep_policy = (params, metrics, out)
+    out.update(mae=metrics[:, 0], rmse=metrics[:, 1], settling_time=metrics[:, 2], energy=metrics[:, 3])
+    return out
 
 
 def base_batch(env):

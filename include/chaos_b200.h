@@ -192,6 +192,36 @@ int cl_step(cl_ctx* ctx, void* stream, const cl_buffers* buf, const cl_io* io);
 int cl_rollout(cl_ctx* ctx, void* stream, const cl_buffers* buf, const cl_io* io,
                const cl_rollout_desc* desc);
 
+/* -- policy evaluation on the device.  Replaces the predict loop of the reference's evaluation
+ *    scripts (code/test_evaluate.py, code/lorenz_pmsm/test_evaluate.py: frozen VecNormalize,
+ *    model.predict(obs, deterministic=True) every step, then the metrics of cl_eval_metrics):
+ *    a stable-baselines3 MlpPolicy (pi = [64, 64], Tanh, linear action_net; float32) runs inside
+ *    the fused rollout of CL_ENV_HR_SYNC / CL_ENV_PMSM_SYNC, one launch for T control intervals.
+ *    Per interval: z = clip((obs - mean) / sqrt(var + epsilon), +-clip_obs) as f32 (skipped when
+ *    obs_mean is NULL) -> a = W3 tanh(W2 tanh(W1 z + b1) + b2) + b3 -> clip to the action box ->
+ *    the env step cl_rollout runs with the same Philox step index.  io / desc carry the optional
+ *    obs / reward / done streams exactly as in cl_rollout; io.action must be NULL.  The metrics use
+ *    err_t = obs components 0..2 after interval t (as the f32 the policy sees next), ctrl_t = the
+ *    clipped action; state, episode counters and the step index advance as in cl_rollout. */
+#define CL_POLICY_HIDDEN 64   /* two hidden layers of this width (SB3 MlpPolicy default) */
+typedef struct cl_policy {
+  const float* params;      /* device f32, torch Linear layout: W1[64][obs_dim] b1[64] W2[64][64] b2[64]
+                               W3[act_dim][64] b3[act_dim] */
+  const double* obs_mean;   /* device f64 [obs_dim]; NULL = no normalisation */
+  const double* obs_var;    /* device f64 [obs_dim] */
+  double epsilon, clip_obs;
+  const float* obs0;        /* device f32: observation interval 0 acts on, obs0[i*obs0_es + c*obs0_cs] */
+  int64_t obs0_es, obs0_cs;
+  float* obs_last;          /* optional device f32, same addressing: observation after the last interval
+                               (may alias obs0) */
+  float* act_out;           /* optional device f32 [T][n][act_dim]: the clipped actions applied */
+  double* metrics;          /* optional device f64 [n][4]: mae, rmse, settling_time, energy */
+  int32_t steady_start;
+  double dt, error_band;
+} cl_policy;
+int cl_policy_rollout(cl_ctx* ctx, void* stream, const cl_buffers* buf, const cl_io* io,
+                      const cl_rollout_desc* desc, const cl_policy* pol);
+
 /* -- derivative helper used by the reference's evaluation script
  *    (code/lorenz_pmsm/test_evaluate.py:105-108 -> PMSM_Sync_Env._get_derivatives,
  *    lorenz_env_try_pmsm.py:51-58; hr_derivatives lorenz_env_try.py:7-12).

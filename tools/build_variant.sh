@@ -11,6 +11,7 @@ S=gym_lorenz_b200/csrc
 nvcc $A -fmad=false "$@" -c $S/tu_parity.cu -o $out/obj_$name/tu_parity.o &
 nvcc $A "$@" -c $S/tu_northstar.cu -o $out/obj_$name/tu_northstar.o &
 nvcc $A -fmad=false "$@" -c $S/tu_rl_ops.cu -o $out/obj_$name/tu_rl_ops.o &
+nvcc $A -fmad=false "$@" -c $S/tu_policy.cu -o $out/obj_$name/tu_policy.o &
 nvcc $A "$@" -c $S/chaos_b200.cu -o $out/obj_$name/chaos_b200.o &
 wait
 nvcc -gencode arch=compute_100a,code=sm_100a -shared -cudart static -o $out/lib_$name.so $out/obj_$name/*.o
