@@ -14,6 +14,8 @@
 #include <math.h>
 #include <stdint.h>
 
+#include <atomic>
+
 #include "../../include/chaos_b200.h"
 
 namespace {
@@ -420,10 +422,27 @@ extern "C" int cl_obs_normalize(void* stream, const float* in, int64_t ies, int6
   if (!in || !out || !mean || !var || dim < 1 || n < 1) return CL_EINVAL;
   const int block = 256;
   const unsigned grid = (unsigned)((n + block - 1) / block);
-  const bool rows = oes == dim && ocs == 1 && (((uintptr_t)out) & 15) == 0 && dim <= 48;
+  // The ROWS transpose needs 32 * dim floats of dynamic shared memory per warp.  Without an opt-in a block
+  // gets 48 KiB in all, and k_normalize<true>'s static sm_mean / sm_std take part of that: the dynamic
+  // allowance is what remains (maxDynamicSharedSizeBytes; dim 47 fits, dim 48 takes the strided kernel).
+  // Only a successful query is kept; after a failed one this call takes the strided kernel, which needs no
+  // shared memory, and the next call asks again.
+  static std::atomic<int64_t> rows_smem_max{-1};
+  int64_t smem_max = rows_smem_max.load(std::memory_order_relaxed);
+  if (smem_max < 0) {
+    cudaFuncAttributes a{};
+    if (cudaFuncGetAttributes(&a, k_normalize<true>) == cudaSuccess) {
+      smem_max = (int64_t)a.maxDynamicSharedSizeBytes;
+      rows_smem_max.store(smem_max, std::memory_order_relaxed);
+    } else {
+      (void)cudaGetLastError();   // a sticky error fails the launch below and is reported there
+    }
+  }
+  const int64_t rows_smem = (int64_t)(block / 32) * 32 * dim * (int64_t)sizeof(float);
+  const bool rows = oes == dim && ocs == 1 && (((uintptr_t)out) & 15) == 0 && rows_smem <= smem_max;
   if (rows)
-    k_normalize<true><<<grid, block, (size_t)(block / 32) * 32 * dim * sizeof(float), (cudaStream_t)stream>>>(
-        in, ies, ics, out, oes, ocs, n, dim, mean, var, epsilon, clip);
+    k_normalize<true><<<grid, block, (size_t)rows_smem, (cudaStream_t)stream>>>(in, ies, ics, out, oes, ocs, n, dim,
+                                                                                mean, var, epsilon, clip);
   else
     k_normalize<false><<<grid, block, 0, (cudaStream_t)stream>>>(in, ies, ics, out, oes, ocs, n, dim, mean, var,
                                                                   epsilon, clip);

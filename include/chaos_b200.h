@@ -365,9 +365,11 @@ int cl_frame_stack_term(void* stream, float* stacked, const float* obs, int64_t 
 
 /* Evaluation metrics of code/lorenz_pmsm/test_evaluate.py:25-59,239-250 for n trajectories at once:
  * err f64 [T][n_err][stride], ctrl f64 [T][n_ctrl][stride] -> out4 f64 [n][4] =
- * (MAE, RMSE over steps >= steady_start averaged over components; settling time = (last step
- * with |e| > error_band, any component) + 1) * dt, NaN if a component never settles... see
- * calculate_advanced_metrics; control energy sum(u^2) * dt). */
+ * (MAE, RMSE over steps >= steady_start averaged over components; settling time = the largest
+ * per-component settling time, np.nanmax as in the reference: a component's is (last step with
+ * |e_c| > error_band) + 1) * dt, 0 if it never leaves the band and NaN if it is outside the band at
+ * the last step; the result is NaN only when every component is; see calculate_advanced_metrics;
+ * control energy sum(u^2) * dt). */
 int cl_eval_metrics(void* stream, const double* err, const double* ctrl, int32_t T, int32_t n_err,
                     int32_t n_ctrl, int64_t n, int64_t stride, int32_t steady_start, double dt,
                     double error_band, double* out4);
