@@ -95,6 +95,14 @@ class Policy(C.Structure):
     ]
 
 
+class Collect(C.Structure):
+    _fields_ = [
+        ("gamma", C.c_double), ("starts", C.c_void_p), ("obs", C.c_void_p), ("actions", C.c_void_p),
+        ("rewards", C.c_void_p), ("values", C.c_void_p), ("log_probs", C.c_void_p),
+        ("episode_starts", C.c_void_p), ("last_values", C.c_void_p),
+    ]
+
+
 class HostView(C.Structure):
     _fields_ = [
         ("obs", C.c_void_p), ("reward", C.c_void_p), ("done", C.c_void_p),
@@ -117,6 +125,8 @@ SYMBOLS = [
     ("cl_rollout", C.c_int, [_VP, _VP, C.POINTER(Buffers), C.POINTER(IO), C.POINTER(RolloutDesc)]),
     ("cl_policy_rollout", C.c_int, [_VP, _VP, C.POINTER(Buffers), C.POINTER(IO), C.POINTER(RolloutDesc),
                                     C.POINTER(Policy)]),
+    ("cl_policy_collect", C.c_int, [_VP, _VP, C.POINTER(Buffers), C.POINTER(IO), C.POINTER(RolloutDesc),
+                                    C.POINTER(Policy), C.POINTER(Collect)]),
     ("cl_derivatives", C.c_int, [_VP, _VP, _VP, _VP, _VP, C.c_int64]),
     ("cl_stats", C.c_int, [_VP, _VP, C.POINTER(Buffers), _VP, C.c_int]),
     ("cl_get_step_index", C.c_int, [_VP, C.POINTER(C.c_uint64)]),

@@ -526,6 +526,38 @@ extern "C" int cl_policy_rollout(cl_ctx* ctx, void* stream, const cl_buffers* bu
   return r;
 }
 
+extern "C" int cl_policy_collect(cl_ctx* ctx, void* stream, const cl_buffers* buf, const cl_io* io,
+                                 const cl_rollout_desc* d, const cl_policy* pol, const cl_collect* col) {
+  if (!ctx) return fail(nullptr, CL_EINVAL, "null ctx");
+  const int kind = ctx->cfg.kind;
+  if (kind != CL_ENV_HR_SYNC && kind != CL_ENV_PMSM_SYNC)
+    return fail(ctx, CL_EINVAL, "cl_policy_collect: env kind %d is not supported (hr_sync and pmsm_sync only)", kind);
+  if (ctx->cfg.flags & CL_F_OBS_F64) return fail(ctx, CL_EINVAL, "cl_policy_collect: float32 observations only");
+  if (!io || !d || !pol || !col || d->T < 1)
+    return fail(ctx, CL_EINVAL, "cl_policy_collect: io/desc/policy/collect required, T >= 1");
+  if (io->action || io->noise) return fail(ctx, CL_EINVAL, "cl_policy_collect: io.action and io.noise must be NULL");
+  if (!pol->params || !pol->obs0) return fail(ctx, CL_EINVAL, "cl_policy_collect: params and obs0 are required");
+  if (pol->act_out || pol->metrics) return fail(ctx, CL_EINVAL, "cl_policy_collect: act_out and metrics must be NULL");
+  if ((pol->obs_mean == nullptr) != (pol->obs_var == nullptr))
+    return fail(ctx, CL_EINVAL, "cl_policy_collect: obs_mean and obs_var go together");
+  if (!col->starts || !col->obs || !col->actions || !col->rewards || !col->values || !col->log_probs ||
+      !col->episode_starts || !col->last_values)
+    return fail(ctx, CL_EINVAL, "cl_policy_collect: starts, the six buffers and last_values are required");
+  KParams p;
+  int r = fill_params(ctx, buf, io, p);
+  if (r) return r;
+  p.T = d->T; p.obs_ts = d->obs_ts; p.rew_ts = d->rew_ts; p.done_ts = d->done_ts;
+  cudaStream_t st = (cudaStream_t)stream;
+  CU(cudaSetDevice(ctx->cfg.device));
+  const cudaError_t e = cl_launch_policy_collect(kind, p, *pol, *col, (float)ctx->lay.act_low,
+                                                 (float)ctx->lay.act_high, st, ctx->sm_count);
+  if (e != cudaSuccess) return fail(ctx, CL_ECUDA, "policy collect launch failed: %s", cudaGetErrorString(e));
+  ctx->launches += 1;
+  r = advance_graph_step(ctx, st, (uint64_t)d->T);
+  if (r == CL_OK) ctx->step_index += (uint64_t)d->T;
+  return r;
+}
+
 extern "C" int64_t cl_dyn_launch_count(const cl_ctx* ctx) { return ctx ? ctx->dyn_launches : 0; }
 extern "C" int64_t cl_plain_launch_count(const cl_ctx* ctx) { return ctx ? ctx->plain_launches : 0; }
 extern "C" int64_t cl_sm_launch_count(const cl_ctx* ctx) { return ctx ? ctx->sm_launches : 0; }

@@ -340,14 +340,23 @@ __device__ __forceinline__ void step_dispatch(typename E::S& s, const KParams& p
   else E::step(s, p, a, nz, obs, rew, term);
 }
 
-template <class E, bool ROLL, bool PLAIN = false, int SPEC = 0, bool RUNPTR = false>
+// What the rollout collector (k_policy_collect) needs of an interval in registers besides the next
+// observation: the reward, the done flags and the pre-reset (terminal) observation it bootstraps from.
+template <class E>
+struct TermOut {
+  typename E::real obs[E::OBS];
+  typename E::real rew;
+  uint32_t dflags;
+};
+
+template <class E, bool ROLL, bool PLAIN = false, int SPEC = 0, bool RUNPTR = false, class TermPtr = decltype(nullptr)>
 __device__ __forceinline__ unsigned env_interval(typename E::S& s, int32_t& ep_len, double& ep_ret,
                                              const KParams& p, const int64_t i, const bool live,
                                              const unsigned lane, const int t, const uint64_t step,
                                              const float* a, const bool want_noise, const bool obs64,
                                              const bool autoreset, unsigned& bad_acc, float* sm_rows, bool& fin,
                                              PlainPending<E>* pend = nullptr, double* blk_stats = nullptr,
-                                             typename E::real* obs_out = nullptr) {
+                                             typename E::real* obs_out = nullptr, TermPtr term_out = nullptr) {
   typedef typename E::real real;
   if (PLAIN && CL_PLAIN_DEFER) plain_emit<E, RUNPTR>(p, i, live, *pend);   // outputs of the previous interval
   // The per-interval Philox stream (key / counter words).  Generic kernels build it up front: building
@@ -429,6 +438,15 @@ __device__ __forceinline__ unsigned env_interval(typename E::S& s, int32_t& ep_l
     // Entries of unfinished envs are not meaningful and never read.
     p.last_ep_ret[i] = ep_ret;
     p.last_ep_len[i] = ep_len;
+  }
+  // before the auto-reset overwrites obs.  term_out is a TermOut<E>* or (every other caller) the default
+  // nullptr: its type removes the copy before code generation (a run-time null test, although folded,
+  // measurably changed the register allocation of k_policy_rollout)
+  if constexpr (!std::is_same<TermPtr, decltype(nullptr)>::value) {
+#pragma unroll
+    for (int c = 0; c < E::OBS; ++c) term_out->obs[c] = obs[c];
+    term_out->rew = rew;
+    term_out->dflags = (uint32_t)((term ? CL_DONE_TERMINATED : 0) | (trunc ? CL_DONE_TRUNCATED : 0));
   }
   if (live && done) {
     if (has_term && !rows_fast) store_obs<real>(p.term_obs, oo, p.obs_es, p.obs_cs, i, obs, E::OBS, obs64);
@@ -1310,4 +1328,6 @@ cudaError_t cl_dyn_occupancy_northstar(int kind, int chunk, int* blocks_per_sm);
 // tu_policy.cu
 cudaError_t cl_launch_policy(int kind, const cl::KParams& p, const cl_policy& q, float act_lo, float act_hi,
                              cudaStream_t st, int sms);
+cudaError_t cl_launch_policy_collect(int kind, const cl::KParams& p, const cl_policy& q, const cl_collect& col,
+                                     float act_lo, float act_hi, cudaStream_t st, int sms);
 cudaError_t cl_fma_peak_launch(int dtype_bytes, int grid, int block, int iters, void* sink, cudaStream_t st);

@@ -30,6 +30,7 @@ enum PhiloxTag : uint32_t {
   TAG_NOISE  = 0x10000000u,  // + block index 0..1 (per-step process noise)
   TAG_ACTION = 0x20000000u,  // synthetic random actions of the fused rollout
   TAG_PARAM  = 0x30000000u,  // per-env parameter randomisation
+  TAG_POLICY = 0x40000000u,  // Gaussian policy noise of the rollout collector (cl_policy_collect)
 };
 
 struct u32x4 { uint32_t x, y, z, w; };

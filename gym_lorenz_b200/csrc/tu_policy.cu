@@ -1,5 +1,7 @@
-// Translation unit of cl_policy_rollout: a trained SB3 MlpPolicy (deterministic actions) fused into the
-// hr_sync / pmsm_sync rollout, with the evaluation metrics of cl_eval_metrics accumulated on the fly.
+// Translation unit of cl_policy_rollout and cl_policy_collect: a trained SB3 MlpPolicy (deterministic
+// actions) fused into the hr_sync / pmsm_sync rollout, with the evaluation metrics of cl_eval_metrics
+// accumulated on the fly; and SB3's collect_rollouts (actor-critic, sampled actions, buffer rows) fused
+// into the same rollout.
 // Built with -fmad=false (see build.py), like tu_parity.cu, so the env arithmetic is bit-identical to
 // cl_rollout's; every fused operation of the policy is an explicit fmaf.
 #include "envs_parity.cuh"
@@ -35,6 +37,66 @@ template <class E> struct WeightArg<E, true> {
 // One thread per env for the whole launch (the MLP costs the same for every env: no task queue).
 // Per control interval: frozen VecNormalize -> MLP (float32, fixed fmaf order) -> clip to the action box
 // -> the same env_interval<E, ROLL> cl_rollout runs, with the same Philox step index -> metrics in f64.
+// z = the observation, or with a frozen normaliser k_normalize's expression: the division stays a division
+// by sqrt(var + eps) (s_sd), computed in f64 and rounded to f32 once
+template <int OBS>
+__device__ __forceinline__ void normalize_obs(const float* ob, float* z, const bool norm, const double* s_mean,
+                                              const double* s_sd, const double clip) {
+#pragma unroll
+  for (int c = 0; c < OBS; ++c) {
+    if (norm) {
+      double v = ((double)ob[c] - s_mean[c]) / s_sd[c];
+      v = v < -clip ? -clip : (v > clip ? clip : v);
+      z[c] = (float)v;
+    } else {
+      z[c] = ob[c];
+    }
+  }
+}
+
+// out = W3 tanh(W2 tanh(W1 z + b1) + b2) + b3 with W in PolicyLayout<OBS, NOUT>: the actor (NOUT = ACT) and
+// the critic (NOUT = 1) of SB3's ActorCriticPolicy.  float32, explicit fmaf in a fixed order.  h1 stays in
+// registers; h2 is produced four units at a time (four independent FMA chains) and folded straight into the
+// output accumulators, so it is never stored.
+template <int OBS, int NOUT>
+__device__ __forceinline__ void mlp_forward(const float* W, const float* z, float* out) {
+  typedef PolicyLayout<OBS, NOUT> LW;
+  const float4* W2v = reinterpret_cast<const float4*>(W + LW::W2);
+  float h1[H];
+#pragma unroll
+  for (int j = 0; j < H; ++j) {
+    float acc = W[LW::B1 + j];
+#pragma unroll
+    for (int c = 0; c < OBS; ++c) acc = fmaf(W[LW::W1 + j * OBS + c], z[c], acc);
+    h1[j] = tanhf(acc);
+  }
+#pragma unroll
+  for (int c = 0; c < NOUT; ++c) out[c] = W[LW::B3 + c];
+#pragma unroll 1
+  for (int j = 0; j < H; j += 4) {
+    float acc[4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) acc[u] = W[LW::B2 + j + u];
+#pragma unroll
+    for (int k4 = 0; k4 < H / 4; ++k4) {
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        const float4 w = W2v[(j + u) * (H / 4) + k4];
+        acc[u] = fmaf(w.x, h1[4 * k4 + 0], acc[u]);
+        acc[u] = fmaf(w.y, h1[4 * k4 + 1], acc[u]);
+        acc[u] = fmaf(w.z, h1[4 * k4 + 2], acc[u]);
+        acc[u] = fmaf(w.w, h1[4 * k4 + 3], acc[u]);
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const float h2 = tanhf(acc[u]);
+#pragma unroll
+      for (int c = 0; c < NOUT; ++c) out[c] = fmaf(W[LW::W3 + c * H + j + u], h2, out[c]);
+    }
+  }
+}
+
 template <class E, bool PARAM>
 __global__ void __launch_bounds__(128, 4) k_policy_rollout(const KParams p, const cl_policy q, const float lo,
                                                            const float hi,
@@ -78,7 +140,6 @@ __global__ void __launch_bounds__(128, 4) k_policy_rollout(const KParams p, cons
   E::prepare(s, p, live);
   const bool autoreset = (p.flags & CL_F_AUTORESET) != 0;
   const bool want_noise = E::NOISE > 0 && E::uses_noise(p);
-  const float4* W2v = reinterpret_cast<const float4*>(W + LW::W2);
 
   // metrics (cl_eval_metrics): sum |e_c| and e_c^2 over t >= steady_start, last t with |e_c| > band, sum |u|^2
   double sa[NERR], sq[NERR], en = 0.0;
@@ -91,52 +152,9 @@ __global__ void __launch_bounds__(128, 4) k_policy_rollout(const KParams p, cons
   const uint64_t step0 = step_base(p);
   for (int t = 0; t < p.T; ++t) {
     float z[OBS];
-#pragma unroll
-    for (int c = 0; c < OBS; ++c) {
-      if (norm) {
-        double v = ((double)ob[c] - s_mean[c]) / s_sd[c];
-        v = v < -q.clip_obs ? -q.clip_obs : (v > q.clip_obs ? q.clip_obs : v);
-        z[c] = (float)v;
-      } else {
-        z[c] = ob[c];
-      }
-    }
-    // h1 stays in registers; h2 is produced four units at a time (four independent FMA chains) and folded
-    // straight into the action accumulators, so it is never stored
-    float h1[H];
-#pragma unroll
-    for (int j = 0; j < H; ++j) {
-      float acc = W[LW::B1 + j];
-#pragma unroll
-      for (int c = 0; c < OBS; ++c) acc = fmaf(W[LW::W1 + j * OBS + c], z[c], acc);
-      h1[j] = tanhf(acc);
-    }
+    normalize_obs<OBS>(ob, z, norm, s_mean, s_sd, q.clip_obs);
     float a[ACT];
-#pragma unroll
-    for (int c = 0; c < ACT; ++c) a[c] = W[LW::B3 + c];
-#pragma unroll 1
-    for (int j = 0; j < H; j += 4) {
-      float acc[4];
-#pragma unroll
-      for (int u = 0; u < 4; ++u) acc[u] = W[LW::B2 + j + u];
-#pragma unroll
-      for (int k4 = 0; k4 < H / 4; ++k4) {
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const float4 w = W2v[(j + u) * (H / 4) + k4];
-          acc[u] = fmaf(w.x, h1[4 * k4 + 0], acc[u]);
-          acc[u] = fmaf(w.y, h1[4 * k4 + 1], acc[u]);
-          acc[u] = fmaf(w.z, h1[4 * k4 + 2], acc[u]);
-          acc[u] = fmaf(w.w, h1[4 * k4 + 3], acc[u]);
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const float h2 = tanhf(acc[u]);
-#pragma unroll
-        for (int c = 0; c < ACT; ++c) a[c] = fmaf(W[LW::W3 + c * H + j + u], h2, a[c]);
-      }
-    }
+    mlp_forward<OBS, ACT>(W, z, a);
 #pragma unroll
     for (int c = 0; c < ACT; ++c) a[c] = clipf(a[c], lo, hi);   // SB3 predict: np.clip to the Box
     if (q.act_out != nullptr && live) {
@@ -189,6 +207,131 @@ __global__ void __launch_bounds__(128, 4) k_policy_rollout(const KParams p, cons
   }
 }
 
+// SB3 OnPolicyAlgorithm.collect_rollouts for an ActorCriticPolicy, one thread per env for the whole launch
+// (arithmetic: include/chaos_b200.h, cl_policy_collect).  Per control interval: frozen VecNormalize ->
+// actor and critic -> Gaussian sample from the TAG_POLICY Philox block of (env, step index) -> log-prob
+// -> the env step of k_policy_rollout -> TimeLimit bootstrap with the critic on the pre-reset
+// observation -> one buffer row.  Shared memory holds the actor block, the critic block (moved to a
+// 16-byte boundary: its V2 rows are read as float4) and log_std.
+template <class E>
+__global__ void __launch_bounds__(128, 4) k_policy_collect(const KParams p, const cl_policy q, const cl_collect col,
+                                                           const float lo, const float hi) {
+  typedef typename E::real real;
+  constexpr int OBS = E::OBS, ACT = E::ACT;
+  typedef PolicyLayout<OBS, ACT> LA;
+  typedef PolicyLayout<OBS, 1> LC;
+  __shared__ __align__(16) float s_w[LA::PADDED + LC::PADDED + ACT];
+  __shared__ double s_mean[OBS], s_sd[OBS];
+  for (int k = threadIdx.x; k < LA::TOTAL; k += blockDim.x) s_w[k] = q.params[k];
+  for (int k = threadIdx.x; k < LC::TOTAL; k += blockDim.x) s_w[LA::PADDED + k] = q.params[LA::TOTAL + k];
+  if (threadIdx.x < ACT) s_w[LA::PADDED + LC::PADDED + threadIdx.x] = q.params[LA::TOTAL + LC::TOTAL + threadIdx.x];
+  const float* WA = s_w;
+  const float* WC = s_w + LA::PADDED;
+  const bool norm = q.obs_mean != nullptr;
+  if (norm && threadIdx.x < OBS) {
+    s_mean[threadIdx.x] = q.obs_mean[threadIdx.x];
+    s_sd[threadIdx.x] = sqrt(q.obs_var[threadIdx.x] + q.epsilon);
+  }
+  __syncthreads();
+
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const bool live = i < p.n;
+  const unsigned lane = threadIdx.x & 31u;
+  typename E::S s = {};
+  int32_t ep_len = 0;
+  double ep_ret = 0.0;
+  float ob[OBS];
+#pragma unroll
+  for (int c = 0; c < OBS; ++c) ob[c] = 0.0f;
+  float start = 0.0f;
+  if (live) {
+    E::load(s, p, i);
+    ep_len = p.ep_len[i];
+    ep_ret = p.ep_return[i];
+#pragma unroll
+    for (int c = 0; c < OBS; ++c) ob[c] = q.obs0[i * q.obs0_es + c * q.obs0_cs];
+    start = col.starts[i];
+  }
+  E::prepare(s, p, live);
+  const bool autoreset = (p.flags & CL_F_AUTORESET) != 0;
+  const bool want_noise = E::NOISE > 0 && E::uses_noise(p);
+  // torch Normal(mu, std).log_prob: std = exp(log_std), log_scale = log(std), var = std^2
+  const float kLogSqrt2Pi = 0.91893853320467274178f;   // (float)log(sqrt(2 pi))
+  float sd[ACT], lsd[ACT], var2[ACT];
+#pragma unroll
+  for (int c = 0; c < ACT; ++c) {
+    sd[c] = expf(s_w[LA::PADDED + LC::PADDED + c]);
+    lsd[c] = logf(sd[c]);
+    var2[c] = 2.0f * (sd[c] * sd[c]);
+  }
+  const float gamma = (float)col.gamma;
+
+  unsigned bad_acc = 0u;
+  bool fin = E::finite(s);
+  const uint64_t step0 = step_base(p);
+  const int64_t n = p.n;
+  for (int t = 0; t < p.T; ++t) {
+    const uint64_t step = step0 + (uint64_t)t;
+    float z[OBS];
+    normalize_obs<OBS>(ob, z, norm, s_mean, s_sd, q.clip_obs);
+    float mu[ACT], v;
+    mlp_forward<OBS, ACT>(WA, z, mu);
+    mlp_forward<OBS, 1>(WC, z, &v);
+    double eps[ACT];
+    draw_normal<ACT>(make_stream(p, i, step), TAG_POLICY, eps);
+    float a[ACT], ac[ACT], lp = 0.0f;
+#pragma unroll
+    for (int c = 0; c < ACT; ++c) {
+      a[c] = fmaf(sd[c], (float)eps[c], mu[c]);
+      const float d = a[c] - mu[c];
+      lp += -(d * d) / var2[c] - lsd[c] - kLogSqrt2Pi;
+      ac[c] = clipf(a[c], lo, hi);   // the env sees the clipped action, the buffer keeps a
+    }
+    real nob[OBS];
+    TermOut<E> tr;
+    env_interval<E, true>(s, ep_len, ep_ret, p, i, live, lane, t, step, ac, want_noise, false, autoreset, bad_acc,
+                          nullptr, fin, nullptr, nullptr, nob, &tr);
+    float r = (float)tr.rew;
+    const bool boot = live && (tr.dflags & CL_DONE_TRUNCATED) && !(tr.dflags & CL_DONE_TERMINATED);
+    if (__any_sync(0xffffffffu, boot)) {   // a TimeLimit truncates whole warps together
+      float ot[OBS], zt[OBS], vt;
+#pragma unroll
+      for (int c = 0; c < OBS; ++c) ot[c] = (float)tr.obs[c];
+      normalize_obs<OBS>(ot, zt, norm, s_mean, s_sd, q.clip_obs);
+      mlp_forward<OBS, 1>(WC, zt, &vt);
+      if (boot) r = r + gamma * vt;
+    }
+    if (live) {
+      const int64_t row = (int64_t)t * n + i;
+#pragma unroll
+      for (int c = 0; c < OBS; ++c) col.obs[row * OBS + c] = z[c];
+#pragma unroll
+      for (int c = 0; c < ACT; ++c) col.actions[row * ACT + c] = a[c];
+      col.rewards[row] = r;
+      col.values[row] = v;
+      col.log_probs[row] = lp;
+      col.episode_starts[row] = start;
+    }
+    start = tr.dflags != 0u ? 1.0f : 0.0f;
+#pragma unroll
+    for (int c = 0; c < OBS; ++c) ob[c] = (float)nob[c];
+  }
+  float z[OBS], v;
+  normalize_obs<OBS>(ob, z, norm, s_mean, s_sd, q.clip_obs);
+  mlp_forward<OBS, 1>(WC, z, &v);
+  if (bad_acc && lane == 0) atomicAdd(&p.stats[CL_STAT_NONFINITE], (double)bad_acc);
+  if (!live) return;
+  col.last_values[i] = v;
+  col.starts[i] = start;
+  E::store(s, p, i);
+  p.ep_len[i] = ep_len;
+  p.ep_return[i] = ep_ret;
+  if (q.obs_last != nullptr) {
+#pragma unroll
+    for (int c = 0; c < OBS; ++c) q.obs_last[i * q.obs0_es + c * q.obs0_cs] = ob[c];
+  }
+}
+
 // Threads of the fullest SM decide the launch: ceil(blocks / SMs) * block, ties -> the larger block (a
 // smaller one stages the weights into shared memory more often: 14 blocks of 32 would not fit one SM).
 int policy_block(int64_t n, int sms) {
@@ -218,6 +361,15 @@ cudaError_t launch_policy(const KParams& p, const cl_policy& q, float lo, float 
   return cudaGetLastError();
 }
 
+template <class E>
+cudaError_t launch_policy_collect(const KParams& p, const cl_policy& q, const cl_collect& col, float lo, float hi,
+                                  cudaStream_t st, int sms) {
+  const int block = policy_block(p.n, sms);
+  const unsigned grid = (unsigned)((p.n + block - 1) / block);
+  k_policy_collect<E><<<grid, block, 0, st>>>(p, q, col, lo, hi);
+  return cudaGetLastError();
+}
+
 }  // namespace
 
 cudaError_t cl_launch_policy(int kind, const KParams& p, const cl_policy& q, float lo, float hi, cudaStream_t st,
@@ -225,6 +377,15 @@ cudaError_t cl_launch_policy(int kind, const KParams& p, const cl_policy& q, flo
   switch (kind) {
     case CL_ENV_HR_SYNC: return launch_policy<EnvHRSync>(p, q, lo, hi, st, sms);
     case CL_ENV_PMSM_SYNC: return launch_policy<EnvPMSMSync>(p, q, lo, hi, st, sms);
+    default: return cudaErrorInvalidValue;
+  }
+}
+
+cudaError_t cl_launch_policy_collect(int kind, const KParams& p, const cl_policy& q, const cl_collect& col, float lo,
+                                     float hi, cudaStream_t st, int sms) {
+  switch (kind) {
+    case CL_ENV_HR_SYNC: return launch_policy_collect<EnvHRSync>(p, q, col, lo, hi, st, sms);
+    case CL_ENV_PMSM_SYNC: return launch_policy_collect<EnvPMSMSync>(p, q, col, lo, hi, st, sms);
     default: return cudaErrorInvalidValue;
   }
 }

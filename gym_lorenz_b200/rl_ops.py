@@ -8,6 +8,7 @@ in csrc/tu_rl_ops.cu.
   eval_metrics(...)      calculate_advanced_metrics + steady-state MAE/RMSE (code/lorenz_pmsm/test_evaluate.py:25-59,239-250)
   evaluate_policy(...)   the predict loop of those scripts + eval_metrics, one launch (csrc/tu_policy.cu)
   DeviceRolloutCollector SB3 OnPolicyAlgorithm.collect_rollouts without NumPy / host round trips
+  FusedRolloutCollector  the same for an SB3 ActorCriticPolicy, the n_steps loop in one launch (csrc/tu_policy.cu)
 """
 from __future__ import annotations
 
@@ -86,6 +87,51 @@ def _policy_kind(kind) -> int:
     return k
 
 
+_SB3_CRITIC_KEYS = ("mlp_extractor.value_net.0.weight", "mlp_extractor.value_net.0.bias",
+                    "mlp_extractor.value_net.2.weight", "mlp_extractor.value_net.2.bias",
+                    "value_net.weight", "value_net.bias", "log_std")
+
+
+def _shapes(k: int, critic: bool):
+    """Parameter shapes of the [64, 64] MlpPolicy for kind k, in packing order."""
+    lay = L.layout(k)
+    obs_dim, act_dim, h = lay.obs_dim, lay.act_dim, L.POLICY_HIDDEN
+    actor = [(h, obs_dim), (h,), (h, h), (h,), (act_dim, h), (act_dim,)]
+    return actor + ([(h, obs_dim), (h,), (h, h), (h,), (1, h), (1,), (act_dim,)] if critic else [])
+
+
+def _read_model_zip(src):
+    """The policy state dict of an SB3 model zip (its `policy.pth` member, read with zipfile and
+    torch.load(weights_only=True): SB3 itself is not needed); any other `src` is returned as is."""
+    if isinstance(src, (str, os.PathLike)):
+        with zipfile.ZipFile(src) as z:
+            if "policy.pth" not in z.namelist():
+                raise ValueError(f"{src}: no policy.pth member (not an SB3 model zip)")
+            return torch.load(BytesIO(z.read("policy.pth")), map_location="cpu", weights_only=True)
+    return src
+
+
+def _sb3_tensors(sd, keys):
+    """The tensors of `keys` from an SB3 policy state dict, refusing missing keys and deeper nets."""
+    missing = [key for key in keys if key not in sd]
+    if missing:
+        raise ValueError(f"not an SB3 MlpPolicy state dict: missing {missing}")
+    for net in ("policy_net", "value_net"):
+        prefix = f"mlp_extractor.{net}."
+        if any(key.startswith(prefix) for key in keys):
+            extra = sorted(key for key in sd if key.startswith(prefix) and key not in keys)
+            if extra:
+                raise ValueError(f"{net} is not [64, 64]: unexpected {extra}")
+    return [sd[key] for key in keys]
+
+
+def _check_shapes(keys, tensors, shapes) -> None:
+    for key, t, shape in zip(keys, tensors, shapes):
+        if t is None or tuple(t.shape) != shape:
+            got = None if t is None else tuple(t.shape)
+            raise ValueError(f"{key}: expected shape {shape}, got {got}")
+
+
 def pack_policy(src, device, kind="hr_sync") -> torch.Tensor:
     """The float32 parameter block `cl_policy_rollout` reads, in torch Linear layout:
     W1[64][obs_dim] b1[64] W2[64][64] b2[64] W3[act_dim][64] b3[act_dim].
@@ -102,13 +148,7 @@ def pack_policy(src, device, kind="hr_sync") -> torch.Tensor:
     architecture; a mismatch raises ValueError before anything reaches the device.
     """
     k = _policy_kind(kind)
-    lay = L.layout(k)
-    obs_dim, act_dim, h = lay.obs_dim, lay.act_dim, L.POLICY_HIDDEN
-    if isinstance(src, (str, os.PathLike)):
-        with zipfile.ZipFile(src) as z:
-            if "policy.pth" not in z.namelist():
-                raise ValueError(f"{src}: no policy.pth member (not an SB3 model zip)")
-            src = torch.load(BytesIO(z.read("policy.pth")), map_location="cpu", weights_only=True)
+    src = _read_model_zip(src)
     if isinstance(src, (tuple, list)):
         if len(src) != 2 or not all(isinstance(m, torch.nn.Module) for m in src):
             raise ValueError("expected a (policy_net, action_net) pair of torch modules")
@@ -120,22 +160,54 @@ def pack_policy(src, device, kind="hr_sync") -> torch.Tensor:
                              "(SB3 MlpPolicy, pi=[64, 64], activation_fn=Tanh)")
         tensors = [leaves[0].weight, leaves[0].bias, leaves[2].weight, leaves[2].bias, anet.weight, anet.bias]
     elif isinstance(src, dict):
-        missing = [key for key in _SB3_KEYS if key not in src]
-        if missing:
-            raise ValueError(f"not an SB3 MlpPolicy state dict: missing {missing}")
-        extra = sorted(key for key in src if key.startswith("mlp_extractor.policy_net.") and key not in _SB3_KEYS)
-        if extra:
-            raise ValueError(f"policy_net is not [64, 64]: unexpected {extra}")
-        tensors = [src[key] for key in _SB3_KEYS]
+        tensors = _sb3_tensors(src, _SB3_KEYS)
     else:
         raise ValueError(f"cannot pack a policy from {type(src).__name__}")
-    shapes = [(h, obs_dim), (h,), (h, h), (h,), (act_dim, h), (act_dim,)]
-    for key, t, shape in zip(_SB3_KEYS, tensors, shapes):
-        if t is None or tuple(t.shape) != shape:
-            got = None if t is None else tuple(t.shape)
-            raise ValueError(f"{key}: expected shape {shape}, got {got}")
+    _check_shapes(_SB3_KEYS, tensors, _shapes(k, critic=False))
     with torch.no_grad():
         return torch.cat([t.detach().reshape(-1).to(torch.float32).cpu() for t in tensors]).to(device)
+
+
+def _n_params(obs_dim: int, act_dim: int, critic: bool) -> int:
+    h = L.POLICY_HIDDEN
+    n = h * (obs_dim + 1 + h + 1 + act_dim) + act_dim
+    return n + (h * (obs_dim + 1 + h + 1 + 1) + 1 + act_dim if critic else 0)
+
+
+def pack_actor_critic(src, device, kind="hr_sync", out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """The float32 parameter block `cl_policy_collect` reads: `pack_policy`'s actor block first, then
+    V1[64][obs_dim] c1[64] V2[64][64] c2[64] Wv[1][64] bv[1] (SB3's `mlp_extractor.value_net` and
+    `value_net`), then log_std[act_dim].  `block[:n_actor]` is a valid `evaluate_policy` block.
+
+    `src` is an SB3 `ActorCriticPolicy` state dict (`pack_policy`'s keys plus
+    `mlp_extractor.value_net.{0,2}.{weight,bias}`, `value_net.{weight,bias}` and `log_std`), the path of
+    an SB3 model zip, or any torch.nn.Module whose `state_dict()` carries those names.  Shapes are
+    checked as in `pack_policy`.  With `out` (a contiguous f32 tensor of the block's size) the block is
+    written in place by device-side copies: no host synchronisation, so a training loop can refresh it
+    after every optimiser step and a captured CUDA graph keeps reading the same storage.
+    """
+    k = _policy_kind(kind)
+    src = _read_model_zip(src)
+    if isinstance(src, torch.nn.Module):
+        src = src.state_dict()
+    if not isinstance(src, dict):
+        raise ValueError(f"cannot pack an actor-critic from {type(src).__name__}")
+    keys = _SB3_KEYS + _SB3_CRITIC_KEYS
+    tensors = _sb3_tensors(src, keys)
+    _check_shapes(keys, tensors, _shapes(k, critic=True))
+    if out is None:
+        with torch.no_grad():
+            return torch.cat([t.detach().reshape(-1).to(torch.float32).cpu() for t in tensors]).to(device)
+    n = sum(t.numel() for t in tensors)
+    if not isinstance(out, torch.Tensor) or out.dtype != torch.float32 or out.numel() != n or \
+            not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous f32 tensor of {n} values")
+    with torch.no_grad():
+        o = 0
+        for t in tensors:
+            out[o:o + t.numel()].view(t.shape).copy_(t.detach(), non_blocking=True)
+            o += t.numel()
+    return out
 
 
 def evaluate_policy(env, policy, T: int, *, normalize=None, dt: Optional[float] = None, error_band: float = 0.05,
@@ -177,7 +249,7 @@ def evaluate_policy(env, policy, T: int, *, normalize=None, dt: Optional[float] 
     if unknown:
         raise ValueError(f"record: unknown streams {unknown}; choose from {_RECORDABLE}")
     params = policy if isinstance(policy, torch.Tensor) else pack_policy(policy, b.device, kind)
-    npar = L.POLICY_HIDDEN * (b.obs_dim + 1 + L.POLICY_HIDDEN + 1 + b.act_dim) + b.act_dim
+    npar = _n_params(b.obs_dim, b.act_dim, critic=False)
     if params.dtype != torch.float32 or params.device != b.device or params.numel() != npar or \
             not params.is_contiguous():
         raise ValueError(f"packed policy must be a contiguous f32 tensor of {npar} values on {b.device}")
@@ -475,3 +547,96 @@ class DeviceRolloutCollector:
                 self._graph_out = self._loop(sync_free=True)
         self._graph.replay()
         return self._graph_out
+
+
+class FusedRolloutCollector:
+    """SB3 `OnPolicyAlgorithm.collect_rollouts` for an `ActorCriticPolicy` (pi = vf = [64, 64], Tanh,
+    Gaussian actions with a state-independent log_std) in ONE launch per rollout (`cl_policy_collect`):
+    per control interval the kernel normalises the observation, runs actor and critic, samples the action
+    from the env's Philox stream (purpose TAG_POLICY), steps the env with the clipped action, bootstraps
+    TimeLimit truncations with the critic on the terminal observation and writes one buffer row.  GAE is
+    `rl_ops.gae` on the result.
+
+    env: a BatchedChaosVecEnv (or device wrapper around one) or a ChaosBatch of kind hr_sync / pmsm_sync.
+    policy: a torch.nn.Module with SB3's parameter names, an SB3 state dict or model zip (see
+    `pack_actor_critic`), or an already packed block.  normalize: a DeviceVecNormalize used frozen (its
+    `obs_rms`, `epsilon`, `clip_obs`); one in training mode or with `norm_reward` is refused -- SB3 would
+    update its statistics every step, which `DeviceRolloutCollector` does.
+
+    `collect()` returns the dict of `DeviceRolloutCollector.collect()` (same keys, shapes, dtypes).  The
+    first call resets the env and starts every episode; later calls continue from the batch's observation
+    planes and the carried `starts`.  `last_values` holds V of the last observation.  `collect()` never
+    synchronises with the host: with the env in graph mode it can be captured in a CUDA graph.
+    `sync_params()` repacks the module's current weights into the same storage (capturable as well).
+    """
+
+    def __init__(self, env, policy, n_steps: int, gamma: float = 0.99, gae_lambda: float = 0.95,
+                 normalize=None):
+        b = env if isinstance(env, ChaosBatch) else base_batch(env)
+        kind = _policy_kind(b.kind)
+        if b.obs_f64:
+            raise ValueError("FusedRolloutCollector needs float32 observations (obs_f64=False)")
+        if int(n_steps) < 1:
+            raise ValueError("n_steps must be >= 1")
+        if normalize is not None and normalize.training:
+            raise ValueError("normalize must be frozen (training=False); DeviceRolloutCollector updates the "
+                             "statistics every step")
+        if normalize is not None and normalize.norm_reward:
+            raise ValueError("reward normalisation is not fused (norm_reward=False); use DeviceRolloutCollector")
+        self.env, self.policy, self.n_steps = env, policy, int(n_steps)
+        self.gamma, self.gae_lambda, self.normalize = gamma, gae_lambda, normalize
+        self.batch, self.kind = b, kind
+        dev, N, T = b.device, b.num_envs, self.n_steps
+        npar = _n_params(b.obs_dim, b.act_dim, critic=True)
+        self.n_actor = _n_params(b.obs_dim, b.act_dim, critic=False)
+        self.params = policy if isinstance(policy, torch.Tensor) else pack_actor_critic(policy, dev, kind)
+        if self.params.dtype != torch.float32 or self.params.device != dev or self.params.numel() != npar or \
+                not self.params.is_contiguous():
+            raise ValueError(f"packed actor-critic must be a contiguous f32 tensor of {npar} values on {dev}")
+        f32 = dict(dtype=torch.float32, device=dev)
+        self.buf = {
+            "obs": torch.empty((T, N, b.obs_dim), **f32),
+            "actions": torch.empty((T, N, b.act_dim), **f32),
+            "rewards": torch.empty((T, N), **f32),
+            "values": torch.empty((T, N), **f32),
+            "log_probs": torch.empty((T, N), **f32),
+            "episode_starts": torch.empty((T, N), **f32),
+        }
+        self.last_values = torch.empty(N, **f32)
+        self.starts = torch.ones(N, **f32)
+        self._started = False
+        self._io = L.IO(last_ep_ret=_p(b.last_ep_ret), last_ep_len=_p(b.last_ep_len))
+        self._desc = L.RolloutDesc(T=T)
+        self._pol = L.Policy(params=_p(self.params), obs0=_p(b.obs_planes), obs0_es=1, obs0_cs=b.n_pad,
+                             obs_last=_p(b.obs_planes))
+        if normalize is not None and normalize.norm_obs:
+            self._pol.obs_mean, self._pol.obs_var = _p(normalize.obs_rms.mean), _p(normalize.obs_rms.var)
+            self._pol.epsilon, self._pol.clip_obs = float(normalize.epsilon), float(normalize.clip_obs)
+        buf = self.buf
+        self._col = L.Collect(gamma=float(gamma), starts=_p(self.starts), obs=_p(buf["obs"]),
+                              actions=_p(buf["actions"]), rewards=_p(buf["rewards"]), values=_p(buf["values"]),
+                              log_probs=_p(buf["log_probs"]), episode_starts=_p(buf["episode_starts"]),
+                              last_values=_p(self.last_values))
+
+    def sync_params(self) -> None:
+        """Repack the policy module's current weights into `self.params` (device copies only)."""
+        if isinstance(self.policy, torch.Tensor):
+            raise ValueError("the collector was given a packed block: there is no module to repack from")
+        pack_actor_critic(self.policy, self.batch.device, self.kind, out=self.params)
+
+    @torch.no_grad()
+    def collect(self) -> Dict[str, torch.Tensor]:
+        b = self.batch
+        if not self._started:
+            b.reset()
+            self.starts.fill_(1.0)
+            self._started = True
+        L.check(b.lib.cl_policy_collect(b.ctx, b._stream(), C.byref(b._bufs), C.byref(self._io),
+                                        C.byref(self._desc), C.byref(self._pol), C.byref(self._col)),
+                b.ctx, "cl_policy_collect")
+        buf = self.buf
+        adv, ret = gae(buf["rewards"], buf["values"], buf["episode_starts"], self.last_values, self.starts,
+                       self.gamma, self.gae_lambda)
+        out = dict(buf)
+        out["advantages"], out["returns"] = adv, ret
+        return out

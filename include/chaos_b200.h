@@ -222,6 +222,43 @@ typedef struct cl_policy {
 int cl_policy_rollout(cl_ctx* ctx, void* stream, const cl_buffers* buf, const cl_io* io,
                       const cl_rollout_desc* desc, const cl_policy* pol);
 
+/* -- rollout collection for PPO / A2C on the device.  Replaces stable-baselines3's
+ *    OnPolicyAlgorithm.collect_rollouts (code/train.py: PPO, n_steps 2048; code/lorenz_pmsm/train.py: A2C)
+ *    for an ActorCriticPolicy (pi = vf = [64, 64], Tanh, Gaussian actions with state-independent
+ *    log_std; float32) on CL_ENV_HR_SYNC / CL_ENV_PMSM_SYNC, one launch for T control intervals.
+ *    pol.params is the actor-critic block: the actor block of cl_policy_rollout first, then
+ *    V1[64][obs_dim] c1[64] V2[64][64] c2[64] Wv[1][64] bv[1], then log_std[act_dim].  pol.act_out and
+ *    pol.metrics must be NULL.  Per interval t, env i (all f32 unless stated):
+ *      1. z = obs, or clip((obs - mean) / sqrt(var + epsilon), +-clip_obs) in f64 rounded to f32 with
+ *         obs_mean set (the frozen VecNormalize of cl_policy_rollout);
+ *      2. mu = W3 tanh(W2 tanh(W1 z + b1) + b2) + b3   (cl_policy_rollout's MLP, explicit fmaf);
+ *      3. V  = Wv tanh(V2 tanh(V1 z + c1) + c2) + bv   (same code, same fmaf order);
+ *      4. eps_c = (float) the f64 Box-Muller normal of Philox block (env id, step index, TAG_POLICY),
+ *         std = expf(log_std), a = fmaf(std, eps, mu);
+ *      5. log_prob = sum_c -(a - mu)^2 / (2 std^2) - log(std) - log(sqrt(2 pi))   (torch Normal.log_prob);
+ *      6. the env step of cl_rollout with clip(a, act_low, act_high) and the same Philox step index;
+ *      7. reward = (float)r; where the step truncated without terminating,
+ *         reward += (float)gamma * V(z_term), z_term the pre-reset observation normalised as in 1;
+ *      8. obs[t][i] = z, actions[t][i] = a (unclipped), rewards[t][i], values[t][i] = V,
+ *         log_probs[t][i], episode_starts[t][i] = starts[i]; then starts[i] = (done flags != 0).
+ *    After the last interval: last_values[i] = V(z of the last observation), starts[i] as carried,
+ *    pol.obs_last (if set) = the last raw observation; state, episode counters, statistics and the
+ *    step index advance as in cl_rollout.  io / desc carry optional obs / reward / done streams as in
+ *    cl_rollout; io.action and io.noise must be NULL.  Buffers are row-major with n = num_envs rows. */
+typedef struct cl_collect {
+  double gamma;
+  float* starts;            /* device f32 [n], in/out: episode starts carried between windows */
+  float* obs;               /* device f32 [T][n][obs_dim] */
+  float* actions;           /* device f32 [T][n][act_dim] */
+  float* rewards;           /* device f32 [T][n] */
+  float* values;            /* device f32 [T][n] */
+  float* log_probs;         /* device f32 [T][n] */
+  float* episode_starts;    /* device f32 [T][n] */
+  float* last_values;       /* device f32 [n] */
+} cl_collect;
+int cl_policy_collect(cl_ctx* ctx, void* stream, const cl_buffers* buf, const cl_io* io,
+                      const cl_rollout_desc* desc, const cl_policy* pol, const cl_collect* col);
+
 /* -- derivative helper used by the reference's evaluation script
  *    (code/lorenz_pmsm/test_evaluate.py:105-108 -> PMSM_Sync_Env._get_derivatives,
  *    lorenz_env_try_pmsm.py:51-58; hr_derivatives lorenz_env_try.py:7-12).
