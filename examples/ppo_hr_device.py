@@ -4,6 +4,9 @@
 GPU: 4,096 envs, DeviceRolloutCollector (CUDA-graph captured), GAE kernel, torch PPO update.
 With --fused the rollouts come from FusedRolloutCollector instead (actor-critic, sampling, env step and
 buffer writes in one kernel launch), whose weights are refreshed from the module after every update.
+With --normalize the env is wrapped in DeviceVecNormalize(norm_reward=False) in training mode, the
+reference's A2C pipeline; with --fused as well the kernel updates the running statistics itself
+(FusedRolloutCollector(update_normalize=True)).
 
 This is a usage example / end-to-end sanity check of the env semantics (episode return must
 improve), not part of the measured hot path.   python examples/ppo_hr_device.py --updates 30
@@ -53,16 +56,20 @@ def main():
     ap.add_argument("--epochs", type=int, default=4)
     ap.add_argument("--minibatches", type=int, default=8)
     ap.add_argument("--fused", action="store_true", help="collect with FusedRolloutCollector (one launch per rollout)")
+    ap.add_argument("--normalize", action="store_true",
+                    help="VecNormalize(norm_reward=False) in training mode around the env")
     args = ap.parse_args()
     torch.manual_seed(0)
     env = BatchedChaosVecEnv("hr_sync", args.envs, seed=0, max_episode_steps=1000)
     pol = ActorCritic().to("cuda:0")
     opt = torch.optim.Adam(pol.parameters(), lr=3e-4)
+    vn = rl_ops.DeviceVecNormalize(env, training=True, norm_reward=False) if args.normalize else None
     if args.fused:
-        col = rl_ops.FusedRolloutCollector(env, pol, n_steps=args.n_steps, gamma=0.99, gae_lambda=0.95)
+        col = rl_ops.FusedRolloutCollector(env, pol, n_steps=args.n_steps, gamma=0.99, gae_lambda=0.95,
+                                           normalize=vn, update_normalize=vn is not None)
     else:
-        col = rl_ops.DeviceRolloutCollector(env, pol, n_steps=args.n_steps, gamma=0.99, gae_lambda=0.95,
-                                            use_cuda_graph=True)
+        col = rl_ops.DeviceRolloutCollector(vn if vn is not None else env, pol, n_steps=args.n_steps, gamma=0.99,
+                                            gae_lambda=0.95, use_cuda_graph=True)
     t0, steps = time.time(), 0
     for it in range(args.updates):
         with torch.no_grad():

@@ -103,6 +103,16 @@ class Collect(C.Structure):
     ]
 
 
+class VecNormUpdate(C.Structure):
+    _fields_ = [
+        ("obs_mean", C.c_void_p), ("obs_var", C.c_void_p), ("obs_count", C.c_void_p),
+        ("ret_mean", C.c_void_p), ("ret_var", C.c_void_p), ("ret_count", C.c_void_p), ("returns", C.c_void_p),
+        ("gamma", C.c_double), ("epsilon", C.c_double), ("clip_obs", C.c_double), ("clip_reward", C.c_double),
+        ("norm_obs", C.c_int32), ("norm_reward", C.c_int32),
+        ("scratch", C.c_void_p), ("scratch_bytes", C.c_int64),
+    ]
+
+
 class HostView(C.Structure):
     _fields_ = [
         ("obs", C.c_void_p), ("reward", C.c_void_p), ("done", C.c_void_p),
@@ -127,6 +137,9 @@ SYMBOLS = [
                                     C.POINTER(Policy)]),
     ("cl_policy_collect", C.c_int, [_VP, _VP, C.POINTER(Buffers), C.POINTER(IO), C.POINTER(RolloutDesc),
                                     C.POINTER(Policy), C.POINTER(Collect)]),
+    ("cl_policy_collect_norm", C.c_int, [_VP, _VP, C.POINTER(Buffers), C.POINTER(IO), C.POINTER(RolloutDesc),
+                                         C.POINTER(Policy), C.POINTER(Collect), C.POINTER(VecNormUpdate)]),
+    ("cl_policy_collect_norm_scratch_bytes", C.c_int, [C.c_int32, C.c_int64, C.POINTER(C.c_int64)]),
     ("cl_derivatives", C.c_int, [_VP, _VP, _VP, _VP, _VP, C.c_int64]),
     ("cl_stats", C.c_int, [_VP, _VP, C.POINTER(Buffers), _VP, C.c_int]),
     ("cl_get_step_index", C.c_int, [_VP, C.POINTER(C.c_uint64)]),

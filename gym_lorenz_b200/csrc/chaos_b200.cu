@@ -558,6 +558,62 @@ extern "C" int cl_policy_collect(cl_ctx* ctx, void* stream, const cl_buffers* bu
   return r;
 }
 
+extern "C" int cl_policy_collect_norm_scratch_bytes(int32_t kind, int64_t n, int64_t* out) {
+  if (kind != CL_ENV_HR_SYNC && kind != CL_ENV_PMSM_SYNC)
+    return fail(nullptr, CL_EINVAL, "cl_policy_collect_norm_scratch_bytes: env kind %d is not supported "
+                "(hr_sync and pmsm_sync only)", kind);
+  if (!out || n < 1) return fail(nullptr, CL_EINVAL, "cl_policy_collect_norm_scratch_bytes: n >= 1 and out required");
+  *out = cl_policy_collect_norm_bytes(kLayouts[kind].obs_dim, n);
+  return CL_OK;
+}
+
+extern "C" int cl_policy_collect_norm(cl_ctx* ctx, void* stream, const cl_buffers* buf, const cl_io* io,
+                                      const cl_rollout_desc* d, const cl_policy* pol, const cl_collect* col,
+                                      const cl_vecnorm_update* vn) {
+  if (!ctx) return fail(nullptr, CL_EINVAL, "null ctx");
+  const int kind = ctx->cfg.kind;
+  if (kind != CL_ENV_HR_SYNC && kind != CL_ENV_PMSM_SYNC)
+    return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: env kind %d is not supported (hr_sync and pmsm_sync only)",
+                kind);
+  if (ctx->cfg.flags & CL_F_OBS_F64) return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: float32 observations only");
+  if (!io || !d || !pol || !col || !vn || d->T < 1)
+    return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: io/desc/policy/collect/vecnorm required, T >= 1");
+  if (io->action || io->noise)
+    return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: io.action and io.noise must be NULL");
+  if (!pol->params || !pol->obs0 || !pol->obs_last)
+    return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: params, obs0 and obs_last are required");
+  if (pol->act_out || pol->metrics)
+    return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: act_out and metrics must be NULL");
+  if (pol->obs_mean || pol->obs_var)
+    return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: pol.obs_mean / obs_var must be NULL (the statistics "
+                "come from the vecnorm argument)");
+  if (!col->starts || !col->obs || !col->actions || !col->rewards || !col->values || !col->log_probs ||
+      !col->episode_starts || !col->last_values)
+    return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: starts, the six buffers and last_values are required");
+  if (!vn->ret_mean || !vn->ret_var || !vn->ret_count || !vn->returns ||
+      (vn->norm_obs && (!vn->obs_mean || !vn->obs_var || !vn->obs_count)))
+    return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: the ret_rms statistics, returns and (norm_obs) the "
+                "obs_rms statistics are required");
+  const int64_t need = cl_policy_collect_norm_bytes(ctx->lay.obs_dim, ctx->cfg.num_envs);
+  if (!vn->scratch || vn->scratch_bytes < need)
+    return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: scratch of %lld bytes required, got %lld", (long long)need,
+                (long long)vn->scratch_bytes);
+  KParams p;
+  int r = fill_params(ctx, buf, io, p);
+  if (r) return r;
+  p.T = d->T; p.obs_ts = d->obs_ts; p.rew_ts = d->rew_ts; p.done_ts = d->done_ts;
+  cudaStream_t st = (cudaStream_t)stream;
+  CU(cudaSetDevice(ctx->cfg.device));
+  const cudaError_t e = cl_launch_policy_collect_norm(kind, p, *pol, *col, *vn, (float)ctx->lay.act_low,
+                                                      (float)ctx->lay.act_high, st, ctx->sm_count);
+  if (e != cudaSuccess)
+    return fail(ctx, CL_ECUDA, "policy collect (training-mode VecNormalize) launch failed: %s", cudaGetErrorString(e));
+  ctx->launches += 1;
+  r = advance_graph_step(ctx, st, (uint64_t)d->T);
+  if (r == CL_OK) ctx->step_index += (uint64_t)d->T;
+  return r;
+}
+
 extern "C" int64_t cl_dyn_launch_count(const cl_ctx* ctx) { return ctx ? ctx->dyn_launches : 0; }
 extern "C" int64_t cl_plain_launch_count(const cl_ctx* ctx) { return ctx ? ctx->plain_launches : 0; }
 extern "C" int64_t cl_sm_launch_count(const cl_ctx* ctx) { return ctx ? ctx->sm_launches : 0; }

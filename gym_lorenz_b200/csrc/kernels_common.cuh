@@ -1330,4 +1330,8 @@ cudaError_t cl_launch_policy(int kind, const cl::KParams& p, const cl_policy& q,
                              cudaStream_t st, int sms);
 cudaError_t cl_launch_policy_collect(int kind, const cl::KParams& p, const cl_policy& q, const cl_collect& col,
                                      float act_lo, float act_hi, cudaStream_t st, int sms);
+cudaError_t cl_launch_policy_collect_norm(int kind, const cl::KParams& p, const cl_policy& q, const cl_collect& col,
+                                          const cl_vecnorm_update& vn, float act_lo, float act_hi, cudaStream_t st,
+                                          int sms);
+int64_t cl_policy_collect_norm_bytes(int obs_dim, int64_t n);
 cudaError_t cl_fma_peak_launch(int dtype_bytes, int grid, int block, int iters, void* sink, cudaStream_t st);

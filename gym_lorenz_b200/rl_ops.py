@@ -560,8 +560,20 @@ class FusedRolloutCollector:
     env: a BatchedChaosVecEnv (or device wrapper around one) or a ChaosBatch of kind hr_sync / pmsm_sync.
     policy: a torch.nn.Module with SB3's parameter names, an SB3 state dict or model zip (see
     `pack_actor_critic`), or an already packed block.  normalize: a DeviceVecNormalize used frozen (its
-    `obs_rms`, `epsilon`, `clip_obs`); one in training mode or with `norm_reward` is refused -- SB3 would
-    update its statistics every step, which `DeviceRolloutCollector` does.
+    `obs_rms`, `epsilon`, `clip_obs`); one in training mode or with `norm_reward` is refused unless
+    `update_normalize=True`.
+
+    update_normalize=True (`cl_policy_collect_norm`): `normalize` is a DeviceVecNormalize in training mode
+    over this batch, with `norm_obs` / `norm_reward` in any combination, and the kernel does what SB3's
+    VecNormalize.step_wait does every step: obs_rms.update on the raw observations, the discounted
+    `returns` (the normaliser's `gamma`) and ret_rms.update, reward normalisation with the updated
+    ret_rms, observations normalised with the updated obs_rms.  `vn.obs_rms`, `vn.ret_rms` and
+    `vn.returns` are updated in place on the device, so a training loop can switch between this collector
+    and `DeviceRolloutCollector` or checkpoint `vn.state_dict()` with continuous statistics.  The first
+    `collect()` starts with `vn.reset_tensor()` (SB3's reset in training mode: obs_rms sees the reset
+    observation, returns are zeroed); `vn.old_obs` is the raw last observation.  The statistics cover the
+    envs of this collector, i.e. one GPU; each interval's batch statistics are summed in a fixed order, so
+    they are bit-reproducible run to run.
 
     `collect()` returns the dict of `DeviceRolloutCollector.collect()` (same keys, shapes, dtypes).  The
     first call resets the env and starts every episode; later calls continue from the batch's observation
@@ -571,18 +583,28 @@ class FusedRolloutCollector:
     """
 
     def __init__(self, env, policy, n_steps: int, gamma: float = 0.99, gae_lambda: float = 0.95,
-                 normalize=None):
+                 normalize=None, update_normalize: bool = False):
         b = env if isinstance(env, ChaosBatch) else base_batch(env)
         kind = _policy_kind(b.kind)
         if b.obs_f64:
             raise ValueError("FusedRolloutCollector needs float32 observations (obs_f64=False)")
         if int(n_steps) < 1:
             raise ValueError("n_steps must be >= 1")
-        if normalize is not None and normalize.training:
-            raise ValueError("normalize must be frozen (training=False); DeviceRolloutCollector updates the "
-                             "statistics every step")
-        if normalize is not None and normalize.norm_reward:
-            raise ValueError("reward normalisation is not fused (norm_reward=False); use DeviceRolloutCollector")
+        self.update_normalize = bool(update_normalize)
+        if self.update_normalize:
+            if normalize is None:
+                raise ValueError("update_normalize=True needs a DeviceVecNormalize (normalize=...)")
+            if not normalize.training:
+                raise ValueError("update_normalize=True needs a normaliser in training mode (training=True)")
+            if base_batch(normalize) is not b or normalize.num_envs != b.num_envs:
+                raise ValueError("update_normalize=True needs a normaliser over this collector's batch")
+        else:
+            if normalize is not None and normalize.training:
+                raise ValueError("normalize must be frozen (training=False); DeviceRolloutCollector updates the "
+                                 "statistics every step, or pass update_normalize=True")
+            if normalize is not None and normalize.norm_reward:
+                raise ValueError("reward normalisation is not fused (norm_reward=False); use DeviceRolloutCollector "
+                                 "or update_normalize=True")
         self.env, self.policy, self.n_steps = env, policy, int(n_steps)
         self.gamma, self.gae_lambda, self.normalize = gamma, gae_lambda, normalize
         self.batch, self.kind = b, kind
@@ -609,7 +631,7 @@ class FusedRolloutCollector:
         self._desc = L.RolloutDesc(T=T)
         self._pol = L.Policy(params=_p(self.params), obs0=_p(b.obs_planes), obs0_es=1, obs0_cs=b.n_pad,
                              obs_last=_p(b.obs_planes))
-        if normalize is not None and normalize.norm_obs:
+        if normalize is not None and normalize.norm_obs and not self.update_normalize:
             self._pol.obs_mean, self._pol.obs_var = _p(normalize.obs_rms.mean), _p(normalize.obs_rms.var)
             self._pol.epsilon, self._pol.clip_obs = float(normalize.epsilon), float(normalize.clip_obs)
         buf = self.buf
@@ -617,6 +639,19 @@ class FusedRolloutCollector:
                               actions=_p(buf["actions"]), rewards=_p(buf["rewards"]), values=_p(buf["values"]),
                               log_probs=_p(buf["log_probs"]), episode_starts=_p(buf["episode_starts"]),
                               last_values=_p(self.last_values))
+        self._vn = None
+        if self.update_normalize:
+            vn = normalize
+            nb = C.c_int64()
+            L.check(b.lib.cl_policy_collect_norm_scratch_bytes(kind, N, C.byref(nb)), None,
+                    "cl_policy_collect_norm_scratch_bytes")
+            self._scratch = torch.empty(nb.value, dtype=torch.uint8, device=dev)
+            self._vn = L.VecNormUpdate(
+                obs_mean=_p(vn.obs_rms.mean), obs_var=_p(vn.obs_rms.var), obs_count=_p(vn.obs_rms.count_t),
+                ret_mean=_p(vn.ret_rms.mean), ret_var=_p(vn.ret_rms.var), ret_count=_p(vn.ret_rms.count_t),
+                returns=_p(vn.returns), gamma=float(vn.gamma), epsilon=float(vn.epsilon),
+                clip_obs=float(vn.clip_obs), clip_reward=float(vn.clip_reward), norm_obs=int(bool(vn.norm_obs)),
+                norm_reward=int(bool(vn.norm_reward)), scratch=_p(self._scratch), scratch_bytes=nb.value)
 
     def sync_params(self) -> None:
         """Repack the policy module's current weights into `self.params` (device copies only)."""
@@ -628,12 +663,21 @@ class FusedRolloutCollector:
     def collect(self) -> Dict[str, torch.Tensor]:
         b = self.batch
         if not self._started:
-            b.reset()
+            if self._vn is not None:
+                self.normalize.reset_tensor()
+            else:
+                b.reset()
             self.starts.fill_(1.0)
             self._started = True
-        L.check(b.lib.cl_policy_collect(b.ctx, b._stream(), C.byref(b._bufs), C.byref(self._io),
-                                        C.byref(self._desc), C.byref(self._pol), C.byref(self._col)),
-                b.ctx, "cl_policy_collect")
+        if self._vn is not None:
+            L.check(b.lib.cl_policy_collect_norm(b.ctx, b._stream(), C.byref(b._bufs), C.byref(self._io),
+                                                 C.byref(self._desc), C.byref(self._pol), C.byref(self._col),
+                                                 C.byref(self._vn)), b.ctx, "cl_policy_collect_norm")
+            self.normalize.old_obs = b._view(b.obs_planes)
+        else:
+            L.check(b.lib.cl_policy_collect(b.ctx, b._stream(), C.byref(b._bufs), C.byref(self._io),
+                                            C.byref(self._desc), C.byref(self._pol), C.byref(self._col)),
+                    b.ctx, "cl_policy_collect")
         buf = self.buf
         adv, ret = gae(buf["rewards"], buf["values"], buf["episode_starts"], self.last_values, self.starts,
                        self.gamma, self.gae_lambda)

@@ -259,6 +259,54 @@ typedef struct cl_collect {
 int cl_policy_collect(cl_ctx* ctx, void* stream, const cl_buffers* buf, const cl_io* io,
                       const cl_rollout_desc* desc, const cl_policy* pol, const cl_collect* col);
 
+/* -- cl_policy_collect behind a VecNormalize in training mode (code/lorenz_pmsm/train.py: A2C through
+ *    VecNormalize(norm_obs=True, norm_reward=False, clip_obs=10), training=True): the running statistics
+ *    are updated inside the launch, as SB3's VecNormalize.step_wait does every step.  One cooperative
+ *    launch; every interval ends with a grid-wide barrier, so the batch statistics of interval t are
+ *    reduced over all n envs before any env normalises its next observation.  The reduction sums the
+ *    per-block partial sums in block order in every block: the result is bit-reproducible run to run.
+ *    Refused, besides what cl_policy_collect refuses: pol.obs_mean set (the statistics come from vn
+ *    alone), pol.obs_last NULL (the raw observation is carried there between intervals), missing
+ *    statistics (obs_* only with norm_obs) or returns, scratch smaller than
+ *    cl_policy_collect_norm_scratch_bytes.  Per interval t, env i, after steps 2-6 of cl_policy_collect
+ *    (actor, critic, sample, log-prob, env step) on z_t:
+ *      1. o = the raw next observation (f32), r = the raw reward, the done flags, o_term = the pre-reset
+ *         observation;
+ *      2. norm_obs: obs_rms.update(o over all n envs) with cl_obs_moments + cl_rms_update's arithmetic:
+ *         f64 sums of (o - mean_old) and (o - mean_old)^2, then the merge of cl_rms_update statement for
+ *         statement; obs_count += n (one f64 addition per interval);
+ *      3. returns[i] = returns[i] * gamma + (double)r (two roundings), then ret_rms.update(returns over
+ *         all n envs) with cl_moments_f64's arithmetic and the same merge -- also with norm_reward = 0;
+ *      4. reward = (float)r, or with norm_reward (float)clip((double)r / sqrt(ret_var + epsilon),
+ *         +-clip_reward), ret_var the updated one; where the step truncated without terminating,
+ *         reward += (float)col.gamma * V(z_term);
+ *      5. z_{t+1} = clip((o - mean) / sqrt(var + epsilon), +-clip_obs) in f64 rounded to f32 with the
+ *         updated obs_rms (z = o without norm_obs); z_term the same of o_term;
+ *      6. returns[i] = 0 where done.
+ *    z_0 is the observation in pol.obs0 normalised with the statistics passed in.  After the last
+ *    interval the statistics and returns hold their updated values, pol.obs_last the last raw
+ *    observation, last_values V(z_T).  io.obs / reward / done, when set, stream the raw env outputs. */
+typedef struct cl_vecnorm_update {
+  double* obs_mean;         /* device f64 [obs_dim], in/out (norm_obs only) */
+  double* obs_var;          /* device f64 [obs_dim], in/out (norm_obs only) */
+  double* obs_count;        /* device f64 [1], in/out (norm_obs only) */
+  double* ret_mean;         /* device f64 [1], in/out */
+  double* ret_var;          /* device f64 [1], in/out */
+  double* ret_count;        /* device f64 [1], in/out */
+  double* returns;          /* device f64 [n], in/out: the discounted returns VecNormalize carries */
+  double gamma, epsilon, clip_obs, clip_reward;
+  int32_t norm_obs, norm_reward;
+  void* scratch;            /* device, caller-owned (nothing is allocated during a CUDA-graph capture) */
+  int64_t scratch_bytes;
+} cl_vecnorm_update;
+int cl_policy_collect_norm(cl_ctx* ctx, void* stream, const cl_buffers* buf, const cl_io* io,
+                           const cl_rollout_desc* desc, const cl_policy* pol, const cl_collect* col,
+                           const cl_vecnorm_update* vn);
+/* scratch cl_policy_collect_norm needs for n envs of `kind` (a function of kind and n alone: it can be
+ * sized without a device): two interval-parity slots of per-block partial sums plus, per env, the raw
+ * reward, done flags and pre-reset observation an interval hands to the next one across the barrier */
+int cl_policy_collect_norm_scratch_bytes(int32_t kind, int64_t n, int64_t* out);
+
 /* -- derivative helper used by the reference's evaluation script
  *    (code/lorenz_pmsm/test_evaluate.py:105-108 -> PMSM_Sync_Env._get_derivatives,
  *    lorenz_env_try_pmsm.py:51-58; hr_derivatives lorenz_env_try.py:7-12).
