@@ -497,71 +497,89 @@ extern "C" int cl_rollout(cl_ctx* ctx, void* stream, const cl_buffers* buf, cons
   return r;
 }
 
+// The fused policy kernels exist for hr_sync and pmsm_sync only.
+static int check_policy_kind(cl_ctx* ctx, const char* fn, int kind) {
+  if (kind == CL_ENV_HR_SYNC || kind == CL_ENV_PMSM_SYNC) return CL_OK;
+  return fail(ctx, CL_EINVAL, "%s: env kind %d is not supported (hr_sync and pmsm_sync only)", fn, kind);
+}
+
+// The refusals the fused policy entry points share, in the order they make them.  fn names the entry point;
+// objs lists the arguments it requires ("io/desc/policy/..."), objs_ok says whether those beyond io / desc /
+// policy are there; with need_last, pol->obs_last is required as well.
+static int policy_prelude(cl_ctx* ctx, const char* fn, const char* objs, bool objs_ok, const cl_io* io,
+                          const cl_rollout_desc* d, const cl_policy* pol, bool need_last) {
+  if (!ctx) return fail(nullptr, CL_EINVAL, "null ctx");
+  const int r = check_policy_kind(ctx, fn, ctx->cfg.kind);
+  if (r) return r;
+  if (ctx->cfg.flags & CL_F_OBS_F64) return fail(ctx, CL_EINVAL, "%s: float32 observations only", fn);
+  if (!io || !d || !pol || !objs_ok || d->T < 1) return fail(ctx, CL_EINVAL, "%s: %s required, T >= 1", fn, objs);
+  if (io->action || io->noise) return fail(ctx, CL_EINVAL, "%s: io.action and io.noise must be NULL", fn);
+  if (!pol->params || !pol->obs0 || (need_last && !pol->obs_last))
+    return fail(ctx, CL_EINVAL, need_last ? "%s: params, obs0 and obs_last are required"
+                                          : "%s: params and obs0 are required", fn);
+  return CL_OK;
+}
+
+// The launch parameters of a fused policy window of d->T intervals, on the context's device.
+static int policy_params(cl_ctx* ctx, const cl_buffers* buf, const cl_io* io, const cl_rollout_desc* d,
+                         KParams& p) {
+  const int r = fill_params(ctx, buf, io, p);
+  if (r) return r;
+  p.T = d->T; p.obs_ts = d->obs_ts; p.rew_ts = d->rew_ts; p.done_ts = d->done_ts;
+  CU(cudaSetDevice(ctx->cfg.device));
+  return CL_OK;
+}
+
+static bool collect_complete(const cl_collect* col) {
+  return col->starts && col->obs && col->actions && col->rewards && col->values && col->log_probs &&
+         col->episode_starts && col->last_values;
+}
+
+// After a fused policy launch: count it and advance the Philox step index by the window's T intervals.
+static int policy_done(cl_ctx* ctx, cudaStream_t st, cudaError_t e, const char* what, int T) {
+  if (e != cudaSuccess) return fail(ctx, CL_ECUDA, "%s launch failed: %s", what, cudaGetErrorString(e));
+  ctx->launches += 1;
+  const int r = advance_graph_step(ctx, st, (uint64_t)T);
+  if (r == CL_OK) ctx->step_index += (uint64_t)T;
+  return r;
+}
+
 extern "C" int cl_policy_rollout(cl_ctx* ctx, void* stream, const cl_buffers* buf, const cl_io* io,
                                  const cl_rollout_desc* d, const cl_policy* pol) {
-  if (!ctx) return fail(nullptr, CL_EINVAL, "null ctx");
-  const int kind = ctx->cfg.kind;
-  if (kind != CL_ENV_HR_SYNC && kind != CL_ENV_PMSM_SYNC)
-    return fail(ctx, CL_EINVAL, "cl_policy_rollout: env kind %d is not supported (hr_sync and pmsm_sync only)", kind);
-  if (ctx->cfg.flags & CL_F_OBS_F64) return fail(ctx, CL_EINVAL, "cl_policy_rollout: float32 observations only");
-  if (!io || !d || !pol || d->T < 1) return fail(ctx, CL_EINVAL, "cl_policy_rollout: io/desc/policy required, T >= 1");
-  if (io->action || io->noise) return fail(ctx, CL_EINVAL, "cl_policy_rollout: io.action and io.noise must be NULL");
-  if (!pol->params || !pol->obs0) return fail(ctx, CL_EINVAL, "cl_policy_rollout: params and obs0 are required");
+  int r = policy_prelude(ctx, "cl_policy_rollout", "io/desc/policy", true, io, d, pol, false);
+  if (r) return r;
   if ((pol->obs_mean == nullptr) != (pol->obs_var == nullptr))
     return fail(ctx, CL_EINVAL, "cl_policy_rollout: obs_mean and obs_var go together");
   if (pol->steady_start < 0 || pol->steady_start >= d->T)
     return fail(ctx, CL_EINVAL, "cl_policy_rollout: steady_start %d outside [0, T)", pol->steady_start);
   KParams p;
-  int r = fill_params(ctx, buf, io, p);
-  if (r) return r;
-  p.T = d->T; p.obs_ts = d->obs_ts; p.rew_ts = d->rew_ts; p.done_ts = d->done_ts;
+  if ((r = policy_params(ctx, buf, io, d, p))) return r;
   cudaStream_t st = (cudaStream_t)stream;
-  CU(cudaSetDevice(ctx->cfg.device));
-  const cudaError_t e = cl_launch_policy(kind, p, *pol, (float)ctx->lay.act_low, (float)ctx->lay.act_high, st,
-                                         ctx->sm_count);
-  if (e != cudaSuccess) return fail(ctx, CL_ECUDA, "policy rollout launch failed: %s", cudaGetErrorString(e));
-  ctx->launches += 1;
-  r = advance_graph_step(ctx, st, (uint64_t)d->T);
-  if (r == CL_OK) ctx->step_index += (uint64_t)d->T;
-  return r;
+  const cudaError_t e = cl_launch_policy(ctx->cfg.kind, p, *pol, (float)ctx->lay.act_low, (float)ctx->lay.act_high,
+                                         st, ctx->sm_count);
+  return policy_done(ctx, st, e, "policy rollout", d->T);
 }
 
 extern "C" int cl_policy_collect(cl_ctx* ctx, void* stream, const cl_buffers* buf, const cl_io* io,
                                  const cl_rollout_desc* d, const cl_policy* pol, const cl_collect* col) {
-  if (!ctx) return fail(nullptr, CL_EINVAL, "null ctx");
-  const int kind = ctx->cfg.kind;
-  if (kind != CL_ENV_HR_SYNC && kind != CL_ENV_PMSM_SYNC)
-    return fail(ctx, CL_EINVAL, "cl_policy_collect: env kind %d is not supported (hr_sync and pmsm_sync only)", kind);
-  if (ctx->cfg.flags & CL_F_OBS_F64) return fail(ctx, CL_EINVAL, "cl_policy_collect: float32 observations only");
-  if (!io || !d || !pol || !col || d->T < 1)
-    return fail(ctx, CL_EINVAL, "cl_policy_collect: io/desc/policy/collect required, T >= 1");
-  if (io->action || io->noise) return fail(ctx, CL_EINVAL, "cl_policy_collect: io.action and io.noise must be NULL");
-  if (!pol->params || !pol->obs0) return fail(ctx, CL_EINVAL, "cl_policy_collect: params and obs0 are required");
+  int r = policy_prelude(ctx, "cl_policy_collect", "io/desc/policy/collect", col != nullptr, io, d, pol, false);
+  if (r) return r;
   if (pol->act_out || pol->metrics) return fail(ctx, CL_EINVAL, "cl_policy_collect: act_out and metrics must be NULL");
   if ((pol->obs_mean == nullptr) != (pol->obs_var == nullptr))
     return fail(ctx, CL_EINVAL, "cl_policy_collect: obs_mean and obs_var go together");
-  if (!col->starts || !col->obs || !col->actions || !col->rewards || !col->values || !col->log_probs ||
-      !col->episode_starts || !col->last_values)
+  if (!collect_complete(col))
     return fail(ctx, CL_EINVAL, "cl_policy_collect: starts, the six buffers and last_values are required");
   KParams p;
-  int r = fill_params(ctx, buf, io, p);
-  if (r) return r;
-  p.T = d->T; p.obs_ts = d->obs_ts; p.rew_ts = d->rew_ts; p.done_ts = d->done_ts;
+  if ((r = policy_params(ctx, buf, io, d, p))) return r;
   cudaStream_t st = (cudaStream_t)stream;
-  CU(cudaSetDevice(ctx->cfg.device));
-  const cudaError_t e = cl_launch_policy_collect(kind, p, *pol, *col, (float)ctx->lay.act_low,
+  const cudaError_t e = cl_launch_policy_collect(ctx->cfg.kind, p, *pol, *col, (float)ctx->lay.act_low,
                                                  (float)ctx->lay.act_high, st, ctx->sm_count);
-  if (e != cudaSuccess) return fail(ctx, CL_ECUDA, "policy collect launch failed: %s", cudaGetErrorString(e));
-  ctx->launches += 1;
-  r = advance_graph_step(ctx, st, (uint64_t)d->T);
-  if (r == CL_OK) ctx->step_index += (uint64_t)d->T;
-  return r;
+  return policy_done(ctx, st, e, "policy collect", d->T);
 }
 
 extern "C" int cl_policy_collect_norm_scratch_bytes(int32_t kind, int64_t n, int64_t* out) {
-  if (kind != CL_ENV_HR_SYNC && kind != CL_ENV_PMSM_SYNC)
-    return fail(nullptr, CL_EINVAL, "cl_policy_collect_norm_scratch_bytes: env kind %d is not supported "
-                "(hr_sync and pmsm_sync only)", kind);
+  const int r = check_policy_kind(nullptr, "cl_policy_collect_norm_scratch_bytes", kind);
+  if (r) return r;
   if (!out || n < 1) return fail(nullptr, CL_EINVAL, "cl_policy_collect_norm_scratch_bytes: n >= 1 and out required");
   *out = cl_policy_collect_norm_bytes(kLayouts[kind].obs_dim, n);
   return CL_OK;
@@ -570,25 +588,15 @@ extern "C" int cl_policy_collect_norm_scratch_bytes(int32_t kind, int64_t n, int
 extern "C" int cl_policy_collect_norm(cl_ctx* ctx, void* stream, const cl_buffers* buf, const cl_io* io,
                                       const cl_rollout_desc* d, const cl_policy* pol, const cl_collect* col,
                                       const cl_vecnorm_update* vn) {
-  if (!ctx) return fail(nullptr, CL_EINVAL, "null ctx");
-  const int kind = ctx->cfg.kind;
-  if (kind != CL_ENV_HR_SYNC && kind != CL_ENV_PMSM_SYNC)
-    return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: env kind %d is not supported (hr_sync and pmsm_sync only)",
-                kind);
-  if (ctx->cfg.flags & CL_F_OBS_F64) return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: float32 observations only");
-  if (!io || !d || !pol || !col || !vn || d->T < 1)
-    return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: io/desc/policy/collect/vecnorm required, T >= 1");
-  if (io->action || io->noise)
-    return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: io.action and io.noise must be NULL");
-  if (!pol->params || !pol->obs0 || !pol->obs_last)
-    return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: params, obs0 and obs_last are required");
+  int r = policy_prelude(ctx, "cl_policy_collect_norm", "io/desc/policy/collect/vecnorm", col && vn, io, d, pol,
+                         true);
+  if (r) return r;
   if (pol->act_out || pol->metrics)
     return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: act_out and metrics must be NULL");
   if (pol->obs_mean || pol->obs_var)
     return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: pol.obs_mean / obs_var must be NULL (the statistics "
                 "come from the vecnorm argument)");
-  if (!col->starts || !col->obs || !col->actions || !col->rewards || !col->values || !col->log_probs ||
-      !col->episode_starts || !col->last_values)
+  if (!collect_complete(col))
     return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: starts, the six buffers and last_values are required");
   if (!vn->ret_mean || !vn->ret_var || !vn->ret_count || !vn->returns ||
       (vn->norm_obs && (!vn->obs_mean || !vn->obs_var || !vn->obs_count)))
@@ -599,19 +607,11 @@ extern "C" int cl_policy_collect_norm(cl_ctx* ctx, void* stream, const cl_buffer
     return fail(ctx, CL_EINVAL, "cl_policy_collect_norm: scratch of %lld bytes required, got %lld", (long long)need,
                 (long long)vn->scratch_bytes);
   KParams p;
-  int r = fill_params(ctx, buf, io, p);
-  if (r) return r;
-  p.T = d->T; p.obs_ts = d->obs_ts; p.rew_ts = d->rew_ts; p.done_ts = d->done_ts;
+  if ((r = policy_params(ctx, buf, io, d, p))) return r;
   cudaStream_t st = (cudaStream_t)stream;
-  CU(cudaSetDevice(ctx->cfg.device));
-  const cudaError_t e = cl_launch_policy_collect_norm(kind, p, *pol, *col, *vn, (float)ctx->lay.act_low,
+  const cudaError_t e = cl_launch_policy_collect_norm(ctx->cfg.kind, p, *pol, *col, *vn, (float)ctx->lay.act_low,
                                                       (float)ctx->lay.act_high, st, ctx->sm_count);
-  if (e != cudaSuccess)
-    return fail(ctx, CL_ECUDA, "policy collect (training-mode VecNormalize) launch failed: %s", cudaGetErrorString(e));
-  ctx->launches += 1;
-  r = advance_graph_step(ctx, st, (uint64_t)d->T);
-  if (r == CL_OK) ctx->step_index += (uint64_t)d->T;
-  return r;
+  return policy_done(ctx, st, e, "policy collect (training-mode VecNormalize)", d->T);
 }
 
 extern "C" int64_t cl_dyn_launch_count(const cl_ctx* ctx) { return ctx ? ctx->dyn_launches : 0; }

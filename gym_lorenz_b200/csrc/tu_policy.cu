@@ -7,21 +7,9 @@
 #include <cooperative_groups.h>
 
 #include "envs_parity.cuh"
+#include "rms_merge.cuh"
 
 using namespace cl;
-
-// Weight placement (A/B in DESIGN.md section 11c): 0 = staged once per block in shared memory and read
-// with warp-uniform broadcast loads; 1 = a __grid_constant__ kernel parameter (constant-bank operands),
-// which needs the weights on the host: the launch then copies them back and synchronises the stream.
-#ifndef CL_POLICY_W_PARAM
-#define CL_POLICY_W_PARAM 0
-#endif
-
-// A/B of the training-mode collector (DESIGN.md section 11e): bit 0 drops the grid barrier, bit 1 the block
-// sums and the cross-block reduction.  Only for timing: any value but 0 computes wrong statistics.
-#ifndef CL_NORM_AB
-#define CL_NORM_AB 0
-#endif
 
 namespace {
 
@@ -35,11 +23,6 @@ struct PolicyLayout {
     TOTAL = B3 + ACT, PADDED = (TOTAL + 3) & ~3
   };
   static_assert(W2 % 4 == 0, "W2 rows are read as float4");
-};
-
-template <class E, bool PARAM> struct WeightArg { struct type { float unused; }; };
-template <class E> struct WeightArg<E, true> {
-  struct type { float w[PolicyLayout<E::OBS, E::ACT>::PADDED]; };
 };
 
 // One thread per env for the whole launch (the MLP costs the same for every env: no task queue).
@@ -105,28 +88,115 @@ __device__ __forceinline__ void mlp_forward(const float* W, const float* z, floa
   }
 }
 
-template <class E, bool PARAM>
+// The frozen normaliser of normalize_obs, set up by threads 0 .. OBS - 1 (k_normalize's expression: the
+// division stays a division by sqrt(var + eps)); s_var, if given, receives var as it is.
+template <int OBS>
+__device__ __forceinline__ void stage_norm(const double* mean, const double* var, const double eps, double* s_mean,
+                                           double* s_sd, double* s_var = nullptr) {
+  if (threadIdx.x < OBS) {
+    s_mean[threadIdx.x] = mean[threadIdx.x];
+    const double v = var[threadIdx.x];
+    if (s_var != nullptr) s_var[threadIdx.x] = v;
+    s_sd[threadIdx.x] = sqrt(v + eps);
+  }
+}
+
+// An actor-critic block (pack_actor_critic) in shared memory: the actor at 0, the critic at LA::PADDED (a
+// 16-byte boundary: its V2 rows are read as float4), log_std after the critic at LA::PADDED + LC::PADDED.
+template <int OBS, int ACT>
+__device__ __forceinline__ void stage_actor_critic(const float* params, float* s_w) {
+  typedef PolicyLayout<OBS, ACT> LA;
+  typedef PolicyLayout<OBS, 1> LC;
+  for (int k = threadIdx.x; k < LA::TOTAL; k += blockDim.x) s_w[k] = params[k];
+  for (int k = threadIdx.x; k < LC::TOTAL; k += blockDim.x) s_w[LA::PADDED + k] = params[LA::TOTAL + k];
+  if (threadIdx.x < ACT) s_w[LA::PADDED + LC::PADDED + threadIdx.x] = params[LA::TOTAL + LC::TOTAL + threadIdx.x];
+}
+
+// SB3's Gaussian action head, torch Normal(mu, std).log_prob with std = exp(log_std), log_scale = log(std),
+// var = std^2.  sample(): a = mu + std * eps (one fmaf), lp = its log-prob summed over the components, ac =
+// a clipped to the action box (the env sees ac, the buffer keeps a).
+template <int ACT>
+struct GaussianHead {
+  float sd[ACT], lsd[ACT], var2[ACT];
+
+  __device__ __forceinline__ explicit GaussianHead(const float* log_std) {
+#pragma unroll
+    for (int c = 0; c < ACT; ++c) {
+      sd[c] = expf(log_std[c]);
+      lsd[c] = logf(sd[c]);
+      var2[c] = 2.0f * (sd[c] * sd[c]);
+    }
+  }
+
+  __device__ __forceinline__ float sample(const float* mu, const double* eps, const float lo, const float hi,
+                                          float* a, float* ac) const {
+    const float kLogSqrt2Pi = 0.91893853320467274178f;   // (float)log(sqrt(2 pi))
+    float lp = 0.0f;
+#pragma unroll
+    for (int c = 0; c < ACT; ++c) {
+      a[c] = fmaf(sd[c], (float)eps[c], mu[c]);
+      const float d = a[c] - mu[c];
+      lp += -(d * d) / var2[c] - lsd[c] - kLogSqrt2Pi;
+      ac[c] = clipf(a[c], lo, hi);
+    }
+    return lp;
+  }
+};
+
+// An env's carried state -- env state, Monitor counters and, if ob is given, the observation it acts on next
+// (cl_policy's obs0 layout) -- loaded from the planes and stored back; store_obs says whether q.obs_last is set.
+template <class E>
+__device__ __forceinline__ void load_env(typename E::S& s, int32_t& ep_len, double& ep_ret, float* ob,
+                                         const KParams& p, const cl_policy& q, const int64_t i) {
+  E::load(s, p, i);
+  ep_len = p.ep_len[i];
+  ep_ret = p.ep_return[i];
+  if (ob != nullptr) {
+#pragma unroll
+    for (int c = 0; c < E::OBS; ++c) ob[c] = q.obs0[i * q.obs0_es + c * q.obs0_cs];
+  }
+}
+
+template <class E>
+__device__ __forceinline__ void store_env(const typename E::S& s, const int32_t ep_len, const double ep_ret,
+                                          const float* ob, const bool store_obs, const KParams& p,
+                                          const cl_policy& q, const int64_t i) {
+  E::store(s, p, i);
+  p.ep_len[i] = ep_len;
+  p.ep_return[i] = ep_ret;
+  if (store_obs) {
+#pragma unroll
+    for (int c = 0; c < E::OBS; ++c) q.obs_last[i * q.obs0_es + c * q.obs0_cs] = ob[c];
+  }
+}
+
+// One row of SB3's RolloutBuffer; the reward r only with_reward (k_policy_collect_norm writes it a pass later).
+template <int OBS, int ACT>
+__device__ __forceinline__ void write_row(const cl_collect& col, const int64_t row, const float* z, const float* a,
+                                          const bool with_reward, const float r, const float v, const float lp,
+                                          const float start) {
+#pragma unroll
+  for (int c = 0; c < OBS; ++c) col.obs[row * OBS + c] = z[c];
+#pragma unroll
+  for (int c = 0; c < ACT; ++c) col.actions[row * ACT + c] = a[c];
+  if (with_reward) col.rewards[row] = r;
+  col.values[row] = v;
+  col.log_probs[row] = lp;
+  col.episode_starts[row] = start;
+}
+
+template <class E>
 __global__ void __launch_bounds__(128, 4) k_policy_rollout(const KParams p, const cl_policy q, const float lo,
-                                                           const float hi,
-                                                           const __grid_constant__ typename WeightArg<E, PARAM>::type wp) {
+                                                           const float hi) {
   typedef typename E::real real;
   constexpr int OBS = E::OBS, ACT = E::ACT, NERR = 3;
   typedef PolicyLayout<OBS, ACT> LW;
-  __shared__ __align__(16) float s_w[PARAM ? 4 : LW::PADDED];
+  __shared__ __align__(16) float s_w[LW::PADDED];
   __shared__ double s_mean[OBS], s_sd[OBS];
-  const float* W;
-  if constexpr (PARAM) {
-    W = wp.w;
-  } else {
-    for (int k = threadIdx.x; k < LW::TOTAL; k += blockDim.x) s_w[k] = q.params[k];
-    W = s_w;
-  }
+  for (int k = threadIdx.x; k < LW::TOTAL; k += blockDim.x) s_w[k] = q.params[k];
+  const float* W = s_w;
   const bool norm = q.obs_mean != nullptr;
-  if (norm && threadIdx.x < OBS) {
-    // k_normalize's expression: the division stays a division by sqrt(var + eps)
-    s_mean[threadIdx.x] = q.obs_mean[threadIdx.x];
-    s_sd[threadIdx.x] = sqrt(q.obs_var[threadIdx.x] + q.epsilon);
-  }
+  if (norm) stage_norm<OBS>(q.obs_mean, q.obs_var, q.epsilon, s_mean, s_sd);
   __syncthreads();
 
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -138,13 +208,7 @@ __global__ void __launch_bounds__(128, 4) k_policy_rollout(const KParams p, cons
   float ob[OBS];
 #pragma unroll
   for (int c = 0; c < OBS; ++c) ob[c] = 0.0f;
-  if (live) {
-    E::load(s, p, i);
-    ep_len = p.ep_len[i];
-    ep_ret = p.ep_return[i];
-#pragma unroll
-    for (int c = 0; c < OBS; ++c) ob[c] = q.obs0[i * q.obs0_es + c * q.obs0_cs];
-  }
+  if (live) load_env<E>(s, ep_len, ep_ret, ob, p, q, i);
   E::prepare(s, p, live);
   const bool autoreset = (p.flags & CL_F_AUTORESET) != 0;
   const bool want_noise = E::NOISE > 0 && E::uses_noise(p);
@@ -187,13 +251,7 @@ __global__ void __launch_bounds__(128, 4) k_policy_rollout(const KParams p, cons
   }
   if (bad_acc && lane == 0) atomicAdd(&p.stats[CL_STAT_NONFINITE], (double)bad_acc);
   if (!live) return;
-  E::store(s, p, i);
-  p.ep_len[i] = ep_len;
-  p.ep_return[i] = ep_ret;
-  if (q.obs_last != nullptr) {
-#pragma unroll
-    for (int c = 0; c < OBS; ++c) q.obs_last[i * q.obs0_es + c * q.obs0_cs] = ob[c];
-  }
+  store_env<E>(s, ep_len, ep_ret, ob, q.obs_last != nullptr, p, q, i);
   if (q.metrics != nullptr) {
     // k_eval_final's combination: averages over components, settling time as np.nanmax over components
     const double m = (double)(p.T - q.steady_start);
@@ -230,16 +288,11 @@ __global__ void __launch_bounds__(128, 4) k_policy_collect(const KParams p, cons
   typedef PolicyLayout<OBS, 1> LC;
   __shared__ __align__(16) float s_w[LA::PADDED + LC::PADDED + ACT];
   __shared__ double s_mean[OBS], s_sd[OBS];
-  for (int k = threadIdx.x; k < LA::TOTAL; k += blockDim.x) s_w[k] = q.params[k];
-  for (int k = threadIdx.x; k < LC::TOTAL; k += blockDim.x) s_w[LA::PADDED + k] = q.params[LA::TOTAL + k];
-  if (threadIdx.x < ACT) s_w[LA::PADDED + LC::PADDED + threadIdx.x] = q.params[LA::TOTAL + LC::TOTAL + threadIdx.x];
+  stage_actor_critic<OBS, ACT>(q.params, s_w);
   const float* WA = s_w;
   const float* WC = s_w + LA::PADDED;
   const bool norm = q.obs_mean != nullptr;
-  if (norm && threadIdx.x < OBS) {
-    s_mean[threadIdx.x] = q.obs_mean[threadIdx.x];
-    s_sd[threadIdx.x] = sqrt(q.obs_var[threadIdx.x] + q.epsilon);
-  }
+  if (norm) stage_norm<OBS>(q.obs_mean, q.obs_var, q.epsilon, s_mean, s_sd);
   __syncthreads();
 
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -253,25 +306,13 @@ __global__ void __launch_bounds__(128, 4) k_policy_collect(const KParams p, cons
   for (int c = 0; c < OBS; ++c) ob[c] = 0.0f;
   float start = 0.0f;
   if (live) {
-    E::load(s, p, i);
-    ep_len = p.ep_len[i];
-    ep_ret = p.ep_return[i];
-#pragma unroll
-    for (int c = 0; c < OBS; ++c) ob[c] = q.obs0[i * q.obs0_es + c * q.obs0_cs];
+    load_env<E>(s, ep_len, ep_ret, ob, p, q, i);
     start = col.starts[i];
   }
   E::prepare(s, p, live);
   const bool autoreset = (p.flags & CL_F_AUTORESET) != 0;
   const bool want_noise = E::NOISE > 0 && E::uses_noise(p);
-  // torch Normal(mu, std).log_prob: std = exp(log_std), log_scale = log(std), var = std^2
-  const float kLogSqrt2Pi = 0.91893853320467274178f;   // (float)log(sqrt(2 pi))
-  float sd[ACT], lsd[ACT], var2[ACT];
-#pragma unroll
-  for (int c = 0; c < ACT; ++c) {
-    sd[c] = expf(s_w[LA::PADDED + LC::PADDED + c]);
-    lsd[c] = logf(sd[c]);
-    var2[c] = 2.0f * (sd[c] * sd[c]);
-  }
+  const GaussianHead<ACT> head(s_w + LA::PADDED + LC::PADDED);
   const float gamma = (float)col.gamma;
 
   unsigned bad_acc = 0u;
@@ -287,14 +328,8 @@ __global__ void __launch_bounds__(128, 4) k_policy_collect(const KParams p, cons
     mlp_forward<OBS, 1>(WC, z, &v);
     double eps[ACT];
     draw_normal<ACT>(make_stream(p, i, step), TAG_POLICY, eps);
-    float a[ACT], ac[ACT], lp = 0.0f;
-#pragma unroll
-    for (int c = 0; c < ACT; ++c) {
-      a[c] = fmaf(sd[c], (float)eps[c], mu[c]);
-      const float d = a[c] - mu[c];
-      lp += -(d * d) / var2[c] - lsd[c] - kLogSqrt2Pi;
-      ac[c] = clipf(a[c], lo, hi);   // the env sees the clipped action, the buffer keeps a
-    }
+    float a[ACT], ac[ACT];
+    const float lp = head.sample(mu, eps, lo, hi, a, ac);
     real nob[OBS];
     TermOut<E> tr;
     env_interval<E, true>(s, ep_len, ep_ret, p, i, live, lane, t, step, ac, want_noise, false, autoreset, bad_acc,
@@ -309,17 +344,7 @@ __global__ void __launch_bounds__(128, 4) k_policy_collect(const KParams p, cons
       mlp_forward<OBS, 1>(WC, zt, &vt);
       if (boot) r = r + gamma * vt;
     }
-    if (live) {
-      const int64_t row = (int64_t)t * n + i;
-#pragma unroll
-      for (int c = 0; c < OBS; ++c) col.obs[row * OBS + c] = z[c];
-#pragma unroll
-      for (int c = 0; c < ACT; ++c) col.actions[row * ACT + c] = a[c];
-      col.rewards[row] = r;
-      col.values[row] = v;
-      col.log_probs[row] = lp;
-      col.episode_starts[row] = start;
-    }
+    if (live) write_row<OBS, ACT>(col, (int64_t)t * n + i, z, a, true, r, v, lp, start);
     start = tr.dflags != 0u ? 1.0f : 0.0f;
 #pragma unroll
     for (int c = 0; c < OBS; ++c) ob[c] = (float)nob[c];
@@ -331,13 +356,7 @@ __global__ void __launch_bounds__(128, 4) k_policy_collect(const KParams p, cons
   if (!live) return;
   col.last_values[i] = v;
   col.starts[i] = start;
-  E::store(s, p, i);
-  p.ep_len[i] = ep_len;
-  p.ep_return[i] = ep_ret;
-  if (q.obs_last != nullptr) {
-#pragma unroll
-    for (int c = 0; c < OBS; ++c) q.obs_last[i * q.obs0_es + c * q.obs0_cs] = ob[c];
-  }
+  store_env<E>(s, ep_len, ep_ret, ob, q.obs_last != nullptr, p, q, i);
 }
 
 // Caller-owned scratch of k_policy_collect_norm, each part on a 256-byte boundary:
@@ -390,17 +409,11 @@ __global__ void __launch_bounds__(128, 4) k_policy_collect_norm(const KParams p,
   __shared__ double s_acc[4][NS];         // per-warp sums of the current interval (blockDim <= 128)
   __shared__ double s_part[4][NS];        // per-warp partial sums of all blocks' slots
   __shared__ double s_tot[NS];
-  for (int k = threadIdx.x; k < LA::TOTAL; k += blockDim.x) s_w[k] = q.params[k];
-  for (int k = threadIdx.x; k < LC::TOTAL; k += blockDim.x) s_w[LA::PADDED + k] = q.params[LA::TOTAL + k];
-  if (threadIdx.x < ACT) s_w[LA::PADDED + LC::PADDED + threadIdx.x] = q.params[LA::TOTAL + LC::TOTAL + threadIdx.x];
+  stage_actor_critic<OBS, ACT>(q.params, s_w);
   const float* WA = s_w;
   const float* WC = s_w + LA::PADDED;
   const bool norm = u.norm_obs != 0, nrew = u.norm_reward != 0;
-  if (norm && threadIdx.x < OBS) {
-    s_mean[threadIdx.x] = u.obs_mean[threadIdx.x];
-    s_var[threadIdx.x] = u.obs_var[threadIdx.x];
-    s_sd[threadIdx.x] = sqrt(s_var[threadIdx.x] + u.epsilon);
-  }
+  if (norm) stage_norm<OBS>(u.obs_mean, u.obs_var, u.epsilon, s_mean, s_sd, s_var);
   if (threadIdx.x == 0) {
     s_ret[0] = *u.ret_mean;
     s_ret[1] = *u.ret_var;
@@ -419,14 +432,7 @@ __global__ void __launch_bounds__(128, 4) k_policy_collect_norm(const KParams p,
   const unsigned lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
   const bool autoreset = (p.flags & CL_F_AUTORESET) != 0;
   const bool want_noise = E::NOISE > 0 && E::uses_noise(p);
-  const float kLogSqrt2Pi = 0.91893853320467274178f;   // (float)log(sqrt(2 pi))
-  float sd[ACT], lsd[ACT], var2[ACT];
-#pragma unroll
-  for (int c = 0; c < ACT; ++c) {
-    sd[c] = expf(s_w[LA::PADDED + LC::PADDED + c]);
-    lsd[c] = logf(sd[c]);
-    var2[c] = 2.0f * (sd[c] * sd[c]);
-  }
+  const GaussianHead<ACT> head(s_w + LA::PADDED + LC::PADDED);
   const float gamma = (float)col.gamma;
   const double bn = (double)n;   // batch count of every update: live envs only
 
@@ -453,6 +459,8 @@ __global__ void __launch_bounds__(128, 4) k_policy_collect_norm(const KParams p,
         } else {
           r = (float)r0;
         }
+        // k_policy_collect's TimeLimit bootstrap.  It stays written out in both kernels: as a shared inline
+        // function it changed the instruction schedule of both.
         const bool boot = live && (f0 & CL_DONE_TRUNCATED) && !(f0 & CL_DONE_TERMINATED);
         if (__any_sync(0xffffffffu, boot)) {
           float ot[OBS], zt[OBS], vt;
@@ -479,9 +487,7 @@ __global__ void __launch_bounds__(128, 4) k_policy_collect_norm(const KParams p,
       double ep_ret = 0.0, ret = 0.0;
       float start = 0.0f;
       if (live) {
-        E::load(s, p, i);
-        ep_len = p.ep_len[i];
-        ep_ret = p.ep_return[i];
+        load_env<E>(s, ep_len, ep_ret, nullptr, p, q, i);
         start = col.starts[i];
         ret = u.returns[i];
       }
@@ -491,14 +497,8 @@ __global__ void __launch_bounds__(128, 4) k_policy_collect_norm(const KParams p,
       mlp_forward<OBS, 1>(WC, z, &v);
       double eps[ACT];
       draw_normal<ACT>(make_stream(p, i, step), TAG_POLICY, eps);
-      float a[ACT], ac[ACT], lp = 0.0f;
-#pragma unroll
-      for (int c = 0; c < ACT; ++c) {
-        a[c] = fmaf(sd[c], (float)eps[c], mu[c]);
-        const float d = a[c] - mu[c];
-        lp += -(d * d) / var2[c] - lsd[c] - kLogSqrt2Pi;
-        ac[c] = clipf(a[c], lo, hi);
-      }
+      float a[ACT], ac[ACT];
+      const float lp = head.sample(mu, eps, lo, hi, a, ac);
       real nob[OBS];
       TermOut<E> tr;
       env_interval<E, true>(s, ep_len, ep_ret, p, i, live, lane, t, step, ac, want_noise, false, autoreset, bad_acc,
@@ -525,25 +525,14 @@ __global__ void __launch_bounds__(128, 4) k_policy_collect_norm(const KParams p,
         if (lane == 0) s_acc[warp][c] += w;
       }
       if (live) {
-        const int64_t row = (int64_t)t * n + i;
-#pragma unroll
-        for (int c = 0; c < OBS; ++c) col.obs[row * OBS + c] = z[c];
-#pragma unroll
-        for (int c = 0; c < ACT; ++c) col.actions[row * ACT + c] = a[c];
-        col.values[row] = v;
-        col.log_probs[row] = lp;
-        col.episode_starts[row] = start;
+        write_row<OBS, ACT>(col, (int64_t)t * n + i, z, a, false, 0.0f, v, lp, start);
         sc.rew[i] = (double)tr.rew;
         sc.flags[i] = tr.dflags;
         if ((tr.dflags & CL_DONE_TRUNCATED) && !(tr.dflags & CL_DONE_TERMINATED)) {
 #pragma unroll
           for (int c = 0; c < OBS; ++c) sc.term[c * n + i] = (float)tr.obs[c];
         }
-        E::store(s, p, i);
-        p.ep_len[i] = ep_len;
-        p.ep_return[i] = ep_ret;
-#pragma unroll
-        for (int c = 0; c < OBS; ++c) q.obs_last[i * q.obs0_es + c * q.obs0_cs] = ob[c];
+        store_env<E>(s, ep_len, ep_ret, ob, true, p, q, i);   // obs_last is required here
         col.starts[i] = tr.dflags != 0u ? 1.0f : 0.0f;
         u.returns[i] = tr.dflags != 0u ? 0.0 : ret;
       }
@@ -555,15 +544,13 @@ __global__ void __launch_bounds__(128, 4) k_policy_collect_norm(const KParams p,
     const unsigned nb = gridDim.x;
     double* slot = sc.slots + (size_t)(t & 1) * NS * nb;   // [NS][blocks]: component-major
     const int nwarp = blockDim.x >> 5;
-    if (CL_NORM_AB & 2) {
-      // A/B: barrier without the reduction
-    } else if (threadIdx.x < NS) {
+    if (threadIdx.x < NS) {
       double a = 0.0;
       for (int w = 0; w < nwarp; ++w) { a += s_acc[w][threadIdx.x]; s_acc[w][threadIdx.x] = 0.0; }
       slot[(size_t)threadIdx.x * nb + blockIdx.x] = a;
     }
-    if (!(CL_NORM_AB & 1)) grid.sync();
-    if (!(CL_NORM_AB & 2)) {
+    grid.sync();
+    {
       // thread j sums blocks j, j + blockDim, ... (NS independent loads in flight), then warp shuffles and the
       // warps in order: the same tree in every block, so every block gets the same bits
       double a[NS];
@@ -586,22 +573,14 @@ __global__ void __launch_bounds__(128, 4) k_policy_collect_norm(const KParams p,
       }
     }
     __syncthreads();
-    // cl_rms_update's merge (k_rms_merge), statement for statement: thread c < OBS feature c, thread OBS ret
+    // cl_rms_update's merge (rms_merge.cuh): thread c < OBS feature c, thread OBS ret
     const int c = threadIdx.x;
     const bool mo = norm && c < OBS, mr = c == OBS;
     if (mo || mr) {
       const double acc1 = mo ? s_tot[c] : s_tot[2 * OBS], acc2 = mo ? s_tot[OBS + c] : s_tot[2 * OBS + 1];
       double* mean = mo ? &s_mean[c] : &s_ret[0];
       double* var = mo ? &s_var[c] : &s_ret[1];
-      const double cnt = mo ? s_cnt[0] : s_cnt[1], tot = cnt + bn;
-      const double d1 = acc1 / bn;
-      const double batch_var = acc2 / bn - d1 * d1;
-      const double batch_mean = *mean + d1;
-      const double delta = batch_mean - *mean;
-      const double new_mean = *mean + delta * bn / tot;
-      const double m2 = *var * cnt + batch_var * bn + delta * delta * cnt * bn / tot;
-      *mean = new_mean;
-      *var = m2 / tot;
+      rms_merge(*mean, *var, mo ? s_cnt[0] : s_cnt[1], bn, acc1, acc2);
       if (mo) s_sd[c] = sqrt(*var + u.epsilon);
       else s_ret[2] = sqrt(*var + u.epsilon);
     }
@@ -633,30 +612,16 @@ int policy_block(int64_t n, int sms) {
   return best;
 }
 
-template <class E>
-cudaError_t launch_policy(const KParams& p, const cl_policy& q, float lo, float hi, cudaStream_t st, int sms) {
-  typedef PolicyLayout<E::OBS, E::ACT> LW;
-  const int block = policy_block(p.n, sms);
-  const unsigned grid = (unsigned)((p.n + block - 1) / block);
-  typename WeightArg<E, CL_POLICY_W_PARAM != 0>::type w;
-  memset(&w, 0, sizeof(w));
-#if CL_POLICY_W_PARAM
-  cudaError_t e = cudaMemcpyAsync(w.w, q.params, sizeof(float) * LW::TOTAL, cudaMemcpyDeviceToHost, st);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-  if (e != cudaSuccess) return e;
-#endif
-  (void)sizeof(LW);
-  k_policy_rollout<E, CL_POLICY_W_PARAM != 0><<<grid, block, 0, st>>>(p, q, lo, hi, w);
-  return cudaGetLastError();
-}
+int64_t grid_for(int64_t n, int block) { return (n + block - 1) / block; }
 
-template <class E>
-cudaError_t launch_policy_collect(const KParams& p, const cl_policy& q, const cl_collect& col, float lo, float hi,
-                                  cudaStream_t st, int sms) {
-  const int block = policy_block(p.n, sms);
-  const unsigned grid = (unsigned)((p.n + block - 1) / block);
-  k_policy_collect<E><<<grid, block, 0, st>>>(p, q, col, lo, hi);
-  return cudaGetLastError();
+// f(EnvHRSync()) or f(EnvPMSMSync()) for the env kind: the policy kernels exist for these two only
+template <class F>
+cudaError_t with_policy_env(int kind, const F& f) {
+  switch (kind) {
+    case CL_ENV_HR_SYNC: return f(EnvHRSync());
+    case CL_ENV_PMSM_SYNC: return f(EnvPMSMSync());
+    default: return cudaErrorInvalidValue;
+  }
 }
 
 // Cooperative: the grid is what the occupancy calculator says is co-resident (blocks per SM x SMs), capped at
@@ -667,7 +632,7 @@ cudaError_t launch_policy_collect_norm(const KParams& p, const cl_policy& q, con
                                        const cl_vecnorm_update& u, float lo, float hi, cudaStream_t st, int sms) {
   int block = policy_block(p.n, sms), per_sm = 0;
   cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_policy_collect_norm<E>, block, 0);
-  if (e == cudaSuccess && block != 128 && (p.n + block - 1) / block > (int64_t)per_sm * sms) {
+  if (e == cudaSuccess && block != 128 && grid_for(p.n, block) > (int64_t)per_sm * sms) {
     // policy_block's grid is not co-resident: 128-thread blocks hold the most envs per SM (the weights in
     // shared memory, not the registers, limit the smaller ones), so the fewest threads own two envs
     block = 128;
@@ -675,7 +640,7 @@ cudaError_t launch_policy_collect_norm(const KParams& p, const cl_policy& q, con
   }
   if (e != cudaSuccess) return e;
   if (per_sm < 1) return cudaErrorCooperativeLaunchTooLarge;
-  const int64_t need = (p.n + block - 1) / block, fit = (int64_t)per_sm * sms;
+  const int64_t need = grid_for(p.n, block), fit = (int64_t)per_sm * sms;
   NormScratch sc;
   norm_scratch(E::OBS, p.n, (char*)u.scratch, &sc);
   cudaLaunchConfig_t cfg = {};
@@ -694,29 +659,27 @@ cudaError_t launch_policy_collect_norm(const KParams& p, const cl_policy& q, con
 
 int64_t cl_policy_collect_norm_bytes(int obs_dim, int64_t n) { return norm_scratch(obs_dim, n, nullptr, nullptr); }
 
-cudaError_t cl_launch_policy_collect_norm(int kind, const KParams& p, const cl_policy& q, const cl_collect& col,
-                                          const cl_vecnorm_update& u, float lo, float hi, cudaStream_t st, int sms) {
-  switch (kind) {
-    case CL_ENV_HR_SYNC: return launch_policy_collect_norm<EnvHRSync>(p, q, col, u, lo, hi, st, sms);
-    case CL_ENV_PMSM_SYNC: return launch_policy_collect_norm<EnvPMSMSync>(p, q, col, u, lo, hi, st, sms);
-    default: return cudaErrorInvalidValue;
-  }
-}
-
 cudaError_t cl_launch_policy(int kind, const KParams& p, const cl_policy& q, float lo, float hi, cudaStream_t st,
                              int sms) {
-  switch (kind) {
-    case CL_ENV_HR_SYNC: return launch_policy<EnvHRSync>(p, q, lo, hi, st, sms);
-    case CL_ENV_PMSM_SYNC: return launch_policy<EnvPMSMSync>(p, q, lo, hi, st, sms);
-    default: return cudaErrorInvalidValue;
-  }
+  return with_policy_env(kind, [&](auto env) {
+    const int block = policy_block(p.n, sms);
+    k_policy_rollout<decltype(env)><<<(unsigned)grid_for(p.n, block), block, 0, st>>>(p, q, lo, hi);
+    return cudaGetLastError();
+  });
 }
 
 cudaError_t cl_launch_policy_collect(int kind, const KParams& p, const cl_policy& q, const cl_collect& col, float lo,
                                      float hi, cudaStream_t st, int sms) {
-  switch (kind) {
-    case CL_ENV_HR_SYNC: return launch_policy_collect<EnvHRSync>(p, q, col, lo, hi, st, sms);
-    case CL_ENV_PMSM_SYNC: return launch_policy_collect<EnvPMSMSync>(p, q, col, lo, hi, st, sms);
-    default: return cudaErrorInvalidValue;
-  }
+  return with_policy_env(kind, [&](auto env) {
+    const int block = policy_block(p.n, sms);
+    k_policy_collect<decltype(env)><<<(unsigned)grid_for(p.n, block), block, 0, st>>>(p, q, col, lo, hi);
+    return cudaGetLastError();
+  });
+}
+
+cudaError_t cl_launch_policy_collect_norm(int kind, const KParams& p, const cl_policy& q, const cl_collect& col,
+                                          const cl_vecnorm_update& u, float lo, float hi, cudaStream_t st, int sms) {
+  return with_policy_env(kind, [&](auto env) {
+    return launch_policy_collect_norm<decltype(env)>(p, q, col, u, lo, hi, st, sms);
+  });
 }

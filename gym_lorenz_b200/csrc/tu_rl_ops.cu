@@ -17,6 +17,7 @@
 #include <atomic>
 
 #include "../../include/chaos_b200.h"
+#include "rms_merge.cuh"
 
 namespace {
 
@@ -386,25 +387,15 @@ extern "C" int cl_moments_f64(void* stream, const double* x, int64_t es, int64_t
   return fail_if(cudaGetLastError());
 }
 
-// Chan et al. parallel update of (mean, var, count) with one batch's shifted sums -- SB3
-// RunningMeanStd.update_from_moments (stable_baselines3/common/running_mean_std.py), the same
-// operations in the same order, entirely on the device: the running count is a device scalar, so
-// a VecNormalize step neither synchronises nor bakes host state into a captured CUDA graph.
+// Chan et al. parallel update of (mean, var, count) with one batch's shifted sums (rms_merge.cuh),
+// entirely on the device: the running count is a device scalar, so a VecNormalize step neither
+// synchronises nor bakes host state into a captured CUDA graph.
 //   acc[0][c] = sum(x - mean_old), acc[1][c] = sum((x - mean_old)^2)   (cl_obs_moments)
 __global__ void k_rms_merge(const double* __restrict__ acc, double n, int dim, double* mean, double* var,
                             double* count) {
   const int c = threadIdx.x;
   const double cnt = *count, tot = cnt + n;
-  if (c < dim) {
-    const double d1 = acc[c] / n;                     // batch_mean - mean
-    const double batch_var = acc[dim + c] / n - d1 * d1;
-    const double batch_mean = mean[c] + d1;
-    const double delta = batch_mean - mean[c];
-    const double new_mean = mean[c] + delta * n / tot;
-    const double m2 = var[c] * cnt + batch_var * n + delta * delta * cnt * n / tot;
-    mean[c] = new_mean;
-    var[c] = m2 / tot;
-  }
+  if (c < dim) rms_merge(mean[c], var[c], cnt, n, acc[c], acc[dim + c]);
   __syncthreads();  // every thread has read *count
   if (c == 0) *count = tot;
 }

@@ -13,6 +13,7 @@ in csrc/tu_rl_ops.cu.
 from __future__ import annotations
 
 import ctypes as C
+import math
 import os
 import zipfile
 from io import BytesIO
@@ -168,10 +169,24 @@ def pack_policy(src, device, kind="hr_sync") -> torch.Tensor:
         return torch.cat([t.detach().reshape(-1).to(torch.float32).cpu() for t in tensors]).to(device)
 
 
-def _n_params(obs_dim: int, act_dim: int, critic: bool) -> int:
-    h = L.POLICY_HIDDEN
-    n = h * (obs_dim + 1 + h + 1 + act_dim) + act_dim
-    return n + (h * (obs_dim + 1 + h + 1 + 1) + 1 + act_dim if critic else 0)
+def _n_params(k: int, critic: bool) -> int:
+    return sum(math.prod(shape) for shape in _shapes(k, critic))
+
+
+def _policy_batch(env, who: str):
+    """The ChaosBatch under `env` and its kind, refusing what the fused policy kernels do not run."""
+    b = env if isinstance(env, ChaosBatch) else base_batch(env)
+    kind = _policy_kind(b.kind)
+    if b.obs_f64:
+        raise ValueError(f"{who} needs float32 observations (obs_f64=False)")
+    return b, kind
+
+
+def _check_packed(params, b, kind: int, critic: bool, what: str) -> None:
+    n = _n_params(kind, critic)
+    if params.dtype != torch.float32 or params.device != b.device or params.numel() != n or \
+            not params.is_contiguous():
+        raise ValueError(f"{what} must be a contiguous f32 tensor of {n} values on {b.device}")
 
 
 def pack_actor_critic(src, device, kind="hr_sync", out: Optional[torch.Tensor] = None) -> torch.Tensor:
@@ -234,10 +249,7 @@ def evaluate_policy(env, policy, T: int, *, normalize=None, dt: Optional[float] 
     The metrics are in observation units.  For hr_sync the error components are err / 50 (the env's
     scale_factor): for state units pass error_band=0.05 / 50 and multiply MAE / RMSE by 50.
     """
-    b = env if isinstance(env, ChaosBatch) else base_batch(env)
-    kind = _policy_kind(b.kind)
-    if b.obs_f64:
-        raise ValueError("evaluate_policy needs float32 observations (obs_f64=False)")
+    b, kind = _policy_batch(env, "evaluate_policy")
     T = int(T)
     if T < 1:
         raise ValueError("T must be >= 1")
@@ -249,10 +261,7 @@ def evaluate_policy(env, policy, T: int, *, normalize=None, dt: Optional[float] 
     if unknown:
         raise ValueError(f"record: unknown streams {unknown}; choose from {_RECORDABLE}")
     params = policy if isinstance(policy, torch.Tensor) else pack_policy(policy, b.device, kind)
-    npar = _n_params(b.obs_dim, b.act_dim, critic=False)
-    if params.dtype != torch.float32 or params.device != b.device or params.numel() != npar or \
-            not params.is_contiguous():
-        raise ValueError(f"packed policy must be a contiguous f32 tensor of {npar} values on {b.device}")
+    _check_packed(params, b, kind, False, "packed policy")
     dev, N, NP = b.device, b.num_envs, b.n_pad
     planes = b._view(b.obs_planes)
     if obs0 is not None:
@@ -584,10 +593,7 @@ class FusedRolloutCollector:
 
     def __init__(self, env, policy, n_steps: int, gamma: float = 0.99, gae_lambda: float = 0.95,
                  normalize=None, update_normalize: bool = False):
-        b = env if isinstance(env, ChaosBatch) else base_batch(env)
-        kind = _policy_kind(b.kind)
-        if b.obs_f64:
-            raise ValueError("FusedRolloutCollector needs float32 observations (obs_f64=False)")
+        b, kind = _policy_batch(env, "FusedRolloutCollector")
         if int(n_steps) < 1:
             raise ValueError("n_steps must be >= 1")
         self.update_normalize = bool(update_normalize)
@@ -609,12 +615,9 @@ class FusedRolloutCollector:
         self.gamma, self.gae_lambda, self.normalize = gamma, gae_lambda, normalize
         self.batch, self.kind = b, kind
         dev, N, T = b.device, b.num_envs, self.n_steps
-        npar = _n_params(b.obs_dim, b.act_dim, critic=True)
-        self.n_actor = _n_params(b.obs_dim, b.act_dim, critic=False)
+        self.n_actor = _n_params(kind, critic=False)
         self.params = policy if isinstance(policy, torch.Tensor) else pack_actor_critic(policy, dev, kind)
-        if self.params.dtype != torch.float32 or self.params.device != dev or self.params.numel() != npar or \
-                not self.params.is_contiguous():
-            raise ValueError(f"packed actor-critic must be a contiguous f32 tensor of {npar} values on {dev}")
+        _check_packed(self.params, b, kind, True, "packed actor-critic")
         f32 = dict(dtype=torch.float32, device=dev)
         self.buf = {
             "obs": torch.empty((T, N, b.obs_dim), **f32),

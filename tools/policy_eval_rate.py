@@ -7,9 +7,8 @@ alternated REPS times and timed with CUDA events:
   eager  -- torch loop: policy (float32 MLP, TF32 off) -> ChaosBatch.step -> err / ctrl stored as f64
             [T][c][N] -> rl_ops.eval_metrics;
   graph  -- the same loop captured as one CUDA graph (env in graph mode) and replayed.
-With --variant-lib (a build with -DCL_POLICY_W_PARAM=1, tools/build_variant.sh) the fused arm is also run with
-the weights as a __grid_constant__ kernel parameter instead of shared memory, alternated with the default build
-in the same process.  Reports env-steps/s and the MLP's algorithmic rate (9,216 flop per env-step) as a share
+With --variant-lib (another build of the library, e.g. from tools/build_variant.sh) the fused arm is also run
+with that build ("fused_variant"), alternated with the default build in the same process.  Reports env-steps/s and the MLP's algorithmic rate (9,216 flop per env-step) as a share
 of the measured FFMA peak (ChaosBatch-independent micro-kernel, measure_fma_peak(dtype_bytes=4)).
 Writes one JSON line per (kind, N, arm) to --out; the GPU name and power limit are read in the same run."""
 import argparse
@@ -102,7 +101,7 @@ def run_case(kind, n, T, reps, var_lib, fma_peak, info):
 
     arms = {"fused": fused, "eager": loop}
     if var_lib is not None:
-        arms["fused_wparam"] = lambda: fused(var_lib)
+        arms["fused_variant"] = lambda: fused(var_lib)
     for fn in arms.values():   # warm-up (module load, cuBLAS heuristics, allocator)
         fn()
     torch.cuda.synchronize()
